@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: DADD patient-conditioned progression (13 MES levels x 50 DDIM steps, lambda = 3, 256x256).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--patients P] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--patients P] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one progression batch per GPU: P patients x 13 levels go through conditioning (AOE + purifier), 50
 CUDA-graph-replayed denoising steps (UNet + fused DDIM) and the VAE decode, producing P*13 images of 256x256.
@@ -20,6 +20,16 @@ After the headline the same run adds (each a separate object of the JSON line):
 ``config5``  the 512x512 stress progression, batch 16 in total split over the ranks;
 ``config3``  the training step (batch 8 per GPU, bf16, 256x256: frozen VAE encode + CLIP, conditioning, UNet forward /
              backward, bucketed gradient all-reduce over NCCL, clip + AdamW), with the all-reduce's exposed share.
+
+``--steps K`` is the number of timed repetitions of every leg: the headline, ``e2e``, ``strong``, ``config4`` (sweeps),
+``config5`` and ``config3`` (training steps); the kernel rooflines time 20 launches each.
+
+``--dump-outputs DIR`` (rank 0) writes what the last timed step returned: ``DIR/images.npy`` (resident inputs) and
+``DIR/e2e_images.npy`` (``sample_progressions``), fp32 (k, 3, 256, 256), the same seeded choice of k images of the batch in
+both, k as large as fits ``DUMP_BYTES`` in all; with ``--impl reference``, ``DIR/eps.npy`` (13, 4, 32, 32) of the last timed
+UNet step and ``DIR/images.npy`` (13, 3, 256, 256) of the timed decode.  Weights and inputs are seeded, and the convolutions
+use cuDNN's heuristic algorithm choice (see ``main``), so two builds run with the same arguments can be compared output for
+output.
 """
 
 from __future__ import annotations
@@ -41,6 +51,7 @@ WORKLOAD = ("13 MES levels x 50 DDIM steps, lambda=3, 256x256, SD-1.x-shaped ran
             "eta=0, VAE decode included")
 UNET_GFLOP_PER_SAMPLE_STEP = 178.7          # SURVEY.md Appendix C.1
 SELF_ATTN_N, SELF_ATTN_D, SELF_ATTN_H = 1024, 40, 8
+DUMP_BYTES = 64_000_000
 
 
 _RESULT_FD = None      # the process's original stdout: carries exactly one JSON line
@@ -124,7 +135,8 @@ class ClockSampler:
 # --------------------------------------------------------------------------------------------------- CPU reference
 def cpu_reference_sample(batch: int, seed: int = 0):
     """A bounded sample of the reference CPU path: ONE UNet denoising step at B = 13 (of the 50) through the oracle
-    port, plus ONE VAE decode at B = 13; returns (seconds_unet_step, seconds_decode, cores)."""
+    port, plus ONE VAE decode at B = 13; returns (unet_step, decode, cores, last): the two timed callables return seconds and
+    leave what they computed in ``last`` ("eps", "images")."""
     import torch
     from oracle import conditioning, unet as ounet, weights
     torch.set_num_threads(os.cpu_count() or 1)
@@ -135,19 +147,20 @@ def cpu_reference_sample(batch: int, seed: int = 0):
     img = torch.randn(1, 16, 768, generator=g).expand(batch, -1, -1).contiguous()
     tgt, src = torch.linspace(0, 3, batch), torch.zeros(batch)
     t = torch.full((batch,), 999, dtype=torch.long)
+    last = {}
     with torch.no_grad():
         cond = conditioning.prepare_conditioning(aw, pw, tgt, src, img)
 
         def unet_step():
             t0 = time.perf_counter()
-            ounet.unet_forward(uw, x, t, cond, ounet.CrossCfg(True, STEER))
+            last["eps"] = ounet.unet_forward(uw, x, t, cond, ounet.CrossCfg(True, STEER))
             return time.perf_counter() - t0
 
         def decode():
             t0 = time.perf_counter()
-            ounet.latents_to_images(vw, x)
+            last["images"] = ounet.latents_to_images(vw, x)
             return time.perf_counter() - t0
-        return unet_step, decode, torch.get_num_threads()
+        return unet_step, decode, torch.get_num_threads(), last
 
 
 def run_reference(args) -> None:
@@ -158,12 +171,14 @@ def run_reference(args) -> None:
     if rank != 0:
         return
     import torch
-    unet_step, decode, cores = cpu_reference_sample(LEVELS)
+    unet_step, decode, cores, last = cpu_reference_sample(LEVELS)
     with torch.no_grad():
         for _ in range(max(1, min(args.warmup, 2))):               # untimed passes (each is ~1 s of host work)
             unet_step()
         t_unet = [unet_step() for _ in range(args.steps)]
         t_dec = decode()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     per_step = statistics.mean(t_unet)
     progression_s = DDIM_STEPS * per_step + t_dec
     value = LEVELS / progression_s
@@ -230,6 +245,19 @@ def parity_block(dev, cdt) -> dict:
 
 
 # --------------------------------------------------------------------------------------------------- B200 arm
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """``out_dir/<name>.npy`` for each tensor of ``arrays`` (all with the same leading batch dimension): fp32, the same seeded
+    choice of batch entries from each, as many as fit ``DUMP_BYTES`` in all."""
+    import numpy as np
+    import torch
+    batch = next(iter(arrays.values())).shape[0]
+    k = min(batch, DUMP_BYTES // sum(t[0].numel() * 4 for t in arrays.values()))
+    pick = torch.randperm(batch, generator=torch.Generator().manual_seed(0))[:k].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t[pick.to(t.device)].float().cpu().numpy())
+
+
 def run_b200(args) -> None:
     import torch
     import progressive_stable_diffusion_b200 as P
@@ -261,9 +289,11 @@ def run_b200(args) -> None:
     d_target = _build_labels(LEVELS, 0.0, 3.0, dev).repeat(patients)
     d_noise = host_noise.to(dev).repeat_interleave(LEVELS, 0)
 
+    last = {}
+
     def step_resident():
         lat = _sample(module, d_target, d_source, d_tokens, d_noise, DDIM_STEPS, dev, 0.0, 1.0, None, STEER, 1.0, False, True)
-        return _latents_to_images(module, lat)
+        last["images"] = _latents_to_images(module, lat)
 
     def step_e2e():
         imgs = sample_progressions(module, host_pixels, host_source, LEVELS, DDIM_STEPS, dev, steer_scale=STEER,
@@ -292,8 +322,12 @@ def run_b200(args) -> None:
         _lib.reset_launch_count()
         seconds = timed(step_resident, args.steps)
         eager_launches = _lib.launch_count()
+        images_resident = last.pop("images")
         seconds_e2e = timed(step_e2e, args.steps)
         clocks = sampler.stop() if sampler else None
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"images": images_resident, "e2e_images": host_images})
+        del images_resident
 
         # ---- dominant kernel, timed live on the launching stream: self-attention N=1024, d=40 at this batch (a kernel timed
         # alone, after a pause that lets the power-capped clocks of the long step recover: the burst peaks are its roofline) ----
@@ -391,11 +425,11 @@ def run_b200(args) -> None:
                 return generate_all(module, jobs, tok16, dev, batch_size=bs4, sampling_steps=DDIM_STEPS, steer_scale=STEER,
                                     rank=rank, world_size=world)
             step_cfg4()
-            sec = timed(step_cfg4, 1)
+            sec = timed(step_cfg4, args.steps) / args.steps
             extras["config4"] = {"workload": "evaluation sweep, ONE of the 5 scales: 50 samples x 4 MES classes = 200 jobs x 50 DDIM steps "
                                              "through generate_all (decode + copy to host included), jobs sharded over the ranks",
                                  "jobs": n_jobs, "batch_per_rank": bs4, "value": n_jobs / sec, "unit": "img/s", "seconds": sec,
-                                 "full_sweep_estimate_s": 5 * sec}
+                                 "timed_sweeps": args.steps, "full_sweep_estimate_s": 5 * sec}
             # ---- config 5: 512x512 (64x64 latents) progression, 16 units in total ----
             if 16 % world == 0:
                 u5 = 16 // world
@@ -411,12 +445,12 @@ def run_b200(args) -> None:
                 try:
                     step_cfg5()
                     step_cfg5()
-                    sec = timed(step_cfg5, 2)
+                    sec = timed(step_cfg5, args.steps)
                 finally:
                     module.cfg.dataset.image_size = 256
                 extras["config5"] = {"workload": "512x512 (64x64x4 latents) progression stress: 16 units x 50 DDIM steps, lambda=3, VAE decode "
                                                  "included; self-attention at N=4096 / 1024 / 256", "units_total": 16, "units_per_gpu": u5,
-                                     "value": 16 * 2 / sec, "unit": "img/s", "ms_per_step": sec / 2 * 1e3}
+                                     "value": 16 * args.steps / sec, "unit": "img/s", "ms_per_step": sec / args.steps * 1e3}
 
     with torch.no_grad():
         if args.profile_step:      # one eager denoising step between cudaProfilerStart/Stop (ncu --profile-from-start off)
@@ -443,8 +477,8 @@ def run_b200(args) -> None:
         for _ in range(2):
             step_train()
         _lib.reset_launch_count()
-        sec_eager = timed(step_train, 3)
-        train_launches = _lib.launch_count() // 3
+        sec_eager = timed(step_train, args.steps)
+        train_launches = _lib.launch_count() // args.steps
         # the whole step (forward, backward, bucket all-reduces, clip, AdamW) as ONE captured graph: the eager step is host-bound
         graphed, why = True, ""
         try:
@@ -452,29 +486,29 @@ def run_b200(args) -> None:
                                                              compute_dtype=torch.bfloat16), generators=(gt,))
             replay()
             torch.cuda.synchronize(dev)
-            sec = timed(replay, 3)
+            sec = timed(replay, args.steps)
         except Exception as e:      # noqa: BLE001 - capture is an optimisation: report and keep the eager number
             graphed, why, sec = False, f"{type(e).__name__}: {e}"[:200], sec_eager
         extras["config3"] = {"workload": "training step, batch 8 per GPU, bf16 compute / fp32 master weights, 256x256: VAE encode + CLIP "
                                          "(frozen), AOE / purifier / resampler, UNet forward + backward, Min-SNR loss, bucketed all-reduce, "
-                                         "clip 1.0, AdamW (4 groups)", "batch_per_gpu": tb, "value": tb * world * 3 / sec, "unit": "img/s",
-                             "ms_per_step": sec / 3 * 1e3, "dadd_launches_per_step": int(train_launches),
+                                         "clip 1.0, AdamW (4 groups)", "batch_per_gpu": tb, "value": tb * world * args.steps / sec, "unit": "img/s",
+                             "ms_per_step": sec / args.steps * 1e3, "dadd_launches_per_step": int(train_launches),
                              "grad_buckets": len(trainer.buckets), "grad_bytes": int(sum(bk.numel for bk in trainer.buckets) * 4),
-                             "cuda_graph": graphed, "ms_per_step_eager": sec_eager / 3 * 1e3}
+                             "cuda_graph": graphed, "ms_per_step_eager": sec_eager / args.steps * 1e3}
         if why:
             extras["config3"]["cuda_graph_error"] = why
         if world > 1:           # exposed share of the gradient all-reduce: the same step with the collective switched off
             if graphed:
                 trainer._skip_allreduce = True
                 replay()
-                sec_off = timed(replay, 3)
+                sec_off = timed(replay, args.steps)
                 trainer._skip_allreduce = False
             else:
                 trainer.world = 1
                 step_train()
-                sec_off = timed(step_train, 3)
+                sec_off = timed(step_train, args.steps)
                 trainer.world = world
-            extras["config3"]["ms_per_step_without_allreduce"] = sec_off / 3 * 1e3
+            extras["config3"]["ms_per_step_without_allreduce"] = sec_off / args.steps * 1e3
             extras["config3"]["allreduce_exposed_share"] = max(0.0, 1.0 - sec_off / sec)
         del trainer
 
@@ -490,7 +524,7 @@ def run_b200(args) -> None:
         return
     if hasattr(os, "sched_setaffinity"):          # undo any affinity narrowing inherited from the communication library
         os.sched_setaffinity(0, range(os.cpu_count() or 1))
-    unet_step, decode, cores = cpu_reference_sample(LEVELS)
+    unet_step, decode, cores, _ = cpu_reference_sample(LEVELS)
     unet_step()
     t_unet, t_dec = unet_step(), decode()
     cpu_progression = DDIM_STEPS * t_unet + t_dec
@@ -540,7 +574,7 @@ def run_b200(args) -> None:
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3, help="timed repetitions of every leg (see above)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--patients", type=int, default=8, help="patient progressions per GPU per step (13 images each)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
@@ -551,11 +585,17 @@ def main() -> None:
     ap.add_argument("--no-extras", action="store_true", help="skip the parity / strong / config4 / config5 legs")
     ap.add_argument("--profile-step", action="store_true",
                     help="after the timed region run ONE eager denoising step inside cudaProfilerStart/Stop (for the ncu launch list)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/*.npy (see above)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # torchrun exports OMP_NUM_THREADS=1 to every rank; rank 0 also times the CPU baseline and needs the host's cores (set before
     # torch is imported).
     if int(os.environ.get("RANK", "0")) == 0:
         os.environ["OMP_NUM_THREADS"] = os.environ["MKL_NUM_THREADS"] = str(os.cpu_count() or 1)
+    # cuDNN's heuristic convolution algorithms, not the ones it times per process: timed picks differ from run to run, and
+    # the rounding differences grow over 50 fp16 denoising steps, so the images of two runs on the same inputs would differ
+    os.environ.setdefault("DADD_CUDNN_BENCHMARK", "0")
     _claim_stdout()
     if args.impl == "reference":
         run_reference(args)

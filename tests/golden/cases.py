@@ -69,6 +69,15 @@ def clip_inputs(kind: str):
     return dims, w, pixels
 
 
+def clip_l14_hidden():
+    """The resamplers' input: ViT-L/14 last hidden states on ``clip_inputs("l14")``, from the oracle tower.  The golden file
+    keeps only a sample of the transformers tower's states, which this reproduces to ~1e-6 relative."""
+    from oracle import image_front_end as fe
+    dims, w, pixels = clip_inputs("l14")
+    with torch.no_grad():
+        return fe.clip_hidden_states(w, pixels, dims["heads"], dims["patch"])[0]
+
+
 def projection_plus_inputs():
     return weights.make_projection_plus_state(seed=6)
 

@@ -1,12 +1,12 @@
-"""Generate golden vectors by running the VERBATIM reference modules (build container only).
+"""Generate golden vectors by running the VERBATIM reference modules of the original project.
 
-    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
+    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py <checkout of umutdundar99/progressive-stable-diffusion>
 
 Imports ``src.models.{feature_purifier,ordinal_embedder,attention_processor_routing_gates,attention_processor_base}``
-from /root/reference (a 3-line ``sys.modules`` shim stands in for the absent ``diffusers`` import, which those files use
+from that checkout (a 3-line ``sys.modules`` shim stands in for the absent ``diffusers`` import, which those files use
 only to name ``AttnProcessor2_0``), loads the seeded weights of ``oracle/weights.py`` into them, runs them on the seeded
-inputs of ``tests/golden/cases.py`` and stores the OUTPUTS as fp32 ``.npz`` next to this file.  /root/reference does not
-exist on the GPU box, so tests only read the committed ``.npz`` files.
+inputs of ``tests/golden/cases.py`` and stores the OUTPUTS as fp32 ``.npz`` next to this file, in the sampled format of
+``tests/golden/store.py``.  The tests only read the committed ``.npz`` files.
 """
 
 from __future__ import annotations
@@ -20,7 +20,9 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
-sys.path.insert(0, "/root/reference")
+if len(sys.argv) != 2 or not os.path.isdir(os.path.join(sys.argv[1], "src", "models")):
+    sys.exit(__doc__)
+sys.path.insert(0, os.path.abspath(sys.argv[1]))
 sys.dont_write_bytecode = True
 
 # shim: the processor files do ``from diffusers.models.attention_processor import AttnProcessor2_0``
@@ -36,6 +38,7 @@ from src.models.feature_purifier import FeaturePurifier  # noqa: E402
 from src.models.ordinal_embedder import AdditiveOrdinalEmbedder  # noqa: E402
 
 from tests.golden import cases  # noqa: E402
+from tests.golden.store import pack  # noqa: E402
 
 
 class _StubAttn(torch.nn.Module):
@@ -94,7 +97,7 @@ def main() -> None:
     out["aoe_delta"] = emb.get_ordinal_delta_embedding(src, labels).numpy()
     out["aoe_delta_same"] = emb.get_ordinal_delta_embedding(labels, labels).numpy()
     out["aoe_table"] = emb._compute_class_table().numpy()
-    np.savez_compressed(os.path.join(HERE, "reference_modules.npz"), **out)
+    np.savez_compressed(os.path.join(HERE, "reference_modules.npz"), **pack(out))
     for k, v in out.items():
         print(k, v.shape, v.dtype)
     # ---- conditioning front end: the REAL transformers CLIP tower + the verbatim reference resamplers -----------
@@ -118,7 +121,7 @@ def main() -> None:
     basic = ImageProjection(clip_embedding_dim=768, cross_attention_dim=768, num_tokens=4)
     basic.load_state_dict(bw)
     fe["projection_basic"] = basic(emb_in).numpy()
-    np.savez_compressed(os.path.join(HERE, "front_end.npz"), **fe)
+    np.savez_compressed(os.path.join(HERE, "front_end.npz"), **pack(fe))
     for k, v in fe.items():
         print(k, v.shape, v.dtype)
 

@@ -3,7 +3,6 @@
 import math
 import os
 
-import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
@@ -12,8 +11,9 @@ pytestmark = pytest.mark.gpu
 
 from oracle import conditioning, processors, sampler  # noqa: E402
 from tests.golden import cases  # noqa: E402
+from tests.golden.store import Golden  # noqa: E402
 
-GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_modules.npz"))
+GOLD = Golden(os.path.join(os.path.dirname(__file__), "golden", "reference_modules.npz"))
 DEV = "cuda:0"
 
 
@@ -514,8 +514,8 @@ def test_cross_attention_processors_vs_reference_golden(case, compute):
     with torch.no_grad():
         out = attn(x.to(DEV), encoder_hidden_states=ehs.to(DEV))
     assert out.dtype == torch.float32
-    ref = torch.from_numpy(GOLD["processor_" + case["name"]])
-    assert rel_err(out, ref) <= (2e-2 if compute == torch.bfloat16 else 4e-3), rel_err(out, ref)
+    got, ref = GOLD.pair("processor_" + case["name"], out)
+    assert rel_err(got, ref) <= (2e-2 if compute == torch.bfloat16 else 4e-3), rel_err(got, ref)
 
 
 def _cross_ref(q, k, v, gates, heads, seg, nseg):
@@ -594,7 +594,7 @@ def test_purifier_matches_reference_golden():
     pur.to(DEV)
     with torch.no_grad():
         out = pur(img.to(DEV), aoe.to(DEV))
-    torch.testing.assert_close(out.cpu(), torch.from_numpy(GOLD["purifier"]), atol=2e-4, rtol=1e-4)
+    torch.testing.assert_close(*GOLD.pair("purifier", out), atol=2e-4, rtol=1e-4)
 
 
 def test_aoe_matches_reference_golden():
@@ -604,11 +604,10 @@ def test_aoe_matches_reference_golden():
     emb.load_state_dict(w)
     emb.to(DEV)
     with torch.no_grad():
-        torch.testing.assert_close(emb(labels.to(DEV)).cpu(), torch.from_numpy(GOLD["aoe_forward"]), atol=2e-5, rtol=1e-4)
-        torch.testing.assert_close(emb.get_negative_embedding(labels.to(DEV)).cpu(), torch.from_numpy(GOLD["aoe_negative"]),
-                                   atol=2e-5, rtol=1e-4)
-        torch.testing.assert_close(emb.get_ordinal_delta_embedding(src.to(DEV), labels.to(DEV)).cpu(),
-                                   torch.from_numpy(GOLD["aoe_delta"]), atol=4e-5, rtol=1e-4)
+        torch.testing.assert_close(*GOLD.pair("aoe_forward", emb(labels.to(DEV))), atol=2e-5, rtol=1e-4)
+        torch.testing.assert_close(*GOLD.pair("aoe_negative", emb.get_negative_embedding(labels.to(DEV))), atol=2e-5, rtol=1e-4)
+        torch.testing.assert_close(*GOLD.pair("aoe_delta", emb.get_ordinal_delta_embedding(src.to(DEV), labels.to(DEV))),
+                                   atol=4e-5, rtol=1e-4)
         same = emb.get_ordinal_delta_embedding(labels.to(DEV), labels.to(DEV))
         assert same.abs().max().item() == 0.0                                           # invariant I1
         # interpolation itself: table + gather + lerp, vs the oracle restatement
@@ -628,7 +627,7 @@ def test_upsample_nearest2x_bit_exact(shape, dtype):
 
 
 # ------------------------------------------------------------------------------------------------ CLIP + resampler front end
-FE = np.load(os.path.join(os.path.dirname(__file__), "golden", "front_end.npz"))
+FE = Golden(os.path.join(os.path.dirname(__file__), "golden", "front_end.npz"))
 
 
 def test_quick_gelu():
@@ -652,7 +651,7 @@ def test_clip_tower_vs_transformers_golden(compute):
     hidden = enc.get_hidden_states(pixels.to(DEV))
     embeds = enc(pixels.to(DEV))
     assert hidden.shape == (2, 257, 1024) and embeds.shape == (2, 768)
-    eh, ee = rel_err(hidden, torch.from_numpy(FE["clip_l14_hidden"])), rel_err(embeds, torch.from_numpy(FE["clip_l14_embeds"]))
+    eh, ee = rel_err(*FE.pair("clip_l14_hidden", hidden)), rel_err(embeds, torch.from_numpy(FE["clip_l14_embeds"]))
     print(f"CLIP ViT-L/14 {compute}: hidden rel err {eh:.4g}, embeds rel err {ee:.4g}")
     tol = 3e-2 if compute == torch.bfloat16 else 5e-3
     assert eh <= tol and ee <= tol, (eh, ee)
@@ -664,14 +663,14 @@ def test_image_projections_vs_reference_golden():
     plus.load_state_dict(cases.projection_plus_inputs(), strict=True)
     plus.to(DEV)
     with torch.no_grad():
-        got = plus(torch.from_numpy(FE["clip_l14_hidden"]).to(DEV))
-    torch.testing.assert_close(got.cpu(), torch.from_numpy(FE["projection_plus"]), atol=2e-3, rtol=1e-3)
+        got = plus(cases.clip_l14_hidden().to(DEV))
+    torch.testing.assert_close(*FE.pair("projection_plus", got), atol=2e-3, rtol=1e-3)
     bw, emb = cases.projection_basic_inputs()
     basic = P.ImageProjection(clip_embedding_dim=768, cross_attention_dim=768, num_tokens=4)
     basic.load_state_dict(bw, strict=True)
     basic.to(DEV)
     with torch.no_grad():
-        torch.testing.assert_close(basic(emb.to(DEV)).cpu(), torch.from_numpy(FE["projection_basic"]), atol=2e-3, rtol=1e-3)
+        torch.testing.assert_close(*FE.pair("projection_basic", basic(emb.to(DEV))), atol=2e-3, rtol=1e-3)
 
 
 def test_module_front_end_from_pixels(compute):
@@ -686,7 +685,7 @@ def test_module_front_end_from_pixels(compute):
     with torch.no_grad():
         tokens = module._get_image_embeds(pixels.to(DEV))
         assert torch.equal(module._get_image_embeds(tokens), tokens)          # projected tokens pass through
-    e = rel_err(tokens, torch.from_numpy(FE["projection_plus"]))
+    e = rel_err(*FE.pair("projection_plus", tokens))
     print(f"front end pixels -> tokens {compute}: rel err {e:.4g}")
     assert e <= (3e-2 if compute == torch.bfloat16 else 5e-3), e
     bare = P.DiffusionModuleWithIP(P.default_config(), build_vae=False)

@@ -1,22 +1,20 @@
 """The oracle restatement vs. outputs of the VERBATIM reference modules (tests/golden/reference_modules.npz,
-made by tests/golden/make_golden.py in the build container)."""
+made by tests/golden/make_golden.py from a checkout of the original project)."""
 
 import os
 
-import numpy as np
 import pytest
 import torch
 
 from oracle import conditioning, processors, weights
 from tests.golden import cases
+from tests.golden.store import Golden
 
-GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_modules.npz"))
+GOLD = Golden(os.path.join(os.path.dirname(__file__), "golden", "reference_modules.npz"))
 
 
 def _close(a: torch.Tensor, name: str, atol=2e-6, rtol=1e-5):
-    ref = torch.from_numpy(GOLD[name])
-    assert a.shape == ref.shape
-    torch.testing.assert_close(a, ref, atol=atol, rtol=rtol)
+    torch.testing.assert_close(*GOLD.pair(name, a), atol=atol, rtol=rtol)
 
 
 @pytest.mark.parametrize("case", cases.PROCESSOR_CASES, ids=lambda c: c["name"])
@@ -27,7 +25,8 @@ def test_processors_match_reference(case):
             out = processors.split_injection_attention(w, x, ehs, case["delta_scale"])
         else:
             out = processors.ordinal_ip_attention(w, x, ehs, case["mode"])
-    _close(out, "processor_" + case["name"], atol=1e-5)
+    # fp32 sums are ordered by the CPU's thread count and vector width: up to 1.7e-5 apart on outputs of magnitude <= 23
+    _close(out, "processor_" + case["name"], atol=3e-5)
 
 
 def test_role_maps_bit_exact():
@@ -55,7 +54,7 @@ def test_aoe_matches_reference():
 
 
 # ---- conditioning front end: oracle vs the real transformers CLIP tower / the verbatim reference resamplers --------------
-FE = np.load(os.path.join(os.path.dirname(__file__), "golden", "front_end.npz"))
+FE = Golden(os.path.join(os.path.dirname(__file__), "golden", "front_end.npz"))
 
 
 def test_clip_oracle_matches_transformers_tiny():
@@ -68,8 +67,9 @@ def test_clip_oracle_matches_transformers_tiny():
 
 def test_projection_oracles_match_reference():
     from oracle import image_front_end as fe
-    hidden = torch.from_numpy(FE["clip_l14_hidden"])
+    hidden = cases.clip_l14_hidden()
+    torch.testing.assert_close(*FE.pair("clip_l14_hidden", hidden), atol=5e-5, rtol=1e-5)      # the resampler's input
     got = fe.projection_plus(cases.projection_plus_inputs(), hidden)
-    torch.testing.assert_close(got, torch.from_numpy(FE["projection_plus"]), atol=5e-5, rtol=1e-5)
+    torch.testing.assert_close(*FE.pair("projection_plus", got), atol=5e-5, rtol=1e-5)
     bw, emb = cases.projection_basic_inputs()
-    torch.testing.assert_close(fe.projection_basic(bw, emb, 4, 768), torch.from_numpy(FE["projection_basic"]), atol=2e-5, rtol=1e-5)
+    torch.testing.assert_close(*FE.pair("projection_basic", fe.projection_basic(bw, emb, 4, 768)), atol=2e-5, rtol=1e-5)

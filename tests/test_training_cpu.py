@@ -19,7 +19,7 @@ from oracle import conditioning, weights  # noqa: E402
 from progressive_stable_diffusion_b200 import training as T  # noqa: E402
 
 
-def test_warmup_cosine_matches_reference_formula():
+def test_warmup_cosine_closed_form():
     # src/models/lr_scheduler.py:41-64: linear from warmup_start_lr over warmup_epochs, then half-cosine to eta_min
     base, start, eta, wu, mx = 1e-4, 1e-6, 1e-6, 5, 100
     assert T.warmup_cosine_lr(0, base, wu, mx, start, eta) == pytest.approx(start)
@@ -28,18 +28,6 @@ def test_warmup_cosine_matches_reference_formula():
     assert T.warmup_cosine_lr(52, base, wu, mx, start, eta) == pytest.approx(eta + (base - eta) * 0.5 * (1 + math.cos(math.pi * 47 / 95)))
     assert T.warmup_cosine_lr(100, base, wu, mx, start, eta) == pytest.approx(eta)
     assert T.warmup_cosine_lr(140, base, wu, mx, start, eta) == pytest.approx(eta)          # progress clamps at 1
-    ref_file = "/root/reference/src/models/lr_scheduler.py"
-    if os.path.exists(ref_file):                                     # build container only: the verbatim scheduler agrees
-        import importlib.util
-        spec = importlib.util.spec_from_file_location("ref_lr_scheduler", ref_file)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        opt = torch.optim.SGD([nn.Parameter(torch.zeros(1))], lr=base)
-        sch = mod.LinearWarmupCosineAnnealingLR(opt, wu, mx, warmup_start_lr=start, eta_min=eta)
-        for epoch in range(0, 110):
-            assert sch.get_last_lr()[0] == pytest.approx(T.warmup_cosine_lr(epoch, base, wu, mx, start, eta), rel=1e-9), epoch
-            opt.step()
-            sch.step()
 
 
 class _Tiny(nn.Module):
