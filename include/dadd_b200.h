@@ -254,7 +254,7 @@ int64_t dadd_minsnr_mse_workspace_bytes(int B);
 int dadd_minsnr_mse(const float* pred, const float* target, const float* weight, float* loss, float* grad,
                     float* workspace, int B, int64_t E, float upstream, void* stream);
 /* Gradient-norm clipping and AdamW over flat fp32 buckets, no host synchronisation:
- * dadd_sumsq writes n_partials partial sums of g^2; dadd_clip_coef turns ALL partials of a step into
+ * dadd_sumsq writes n_partials partial sums of g^2 (g may be NULL when n == 0); dadd_clip_coef turns ALL partials of a step into
  * coef_and_norm[0] = grad_scale * min(1, max_norm / (norm + 1e-6)) (max_norm <= 0: no clipping) and [1] = norm =
  * grad_scale * sqrt(sum) (torch.nn.utils.clip_grad_norm_; grad_scale = 1 / world size when the buckets hold SUMS);
  * dadd_adamw_step applies torch.optim.AdamW's update with g scaled by coef[0] (coef may be NULL).  A non-finite norm (fp16
@@ -264,8 +264,10 @@ int dadd_clip_coef(const float* partials, int n, float max_norm, float grad_scal
 int dadd_adamw_step(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2, float eps,
                     float weight_decay, float bias_corr1, float bias_corr2, const float* coef, void* stream);
 /* The same update with the step-dependent scalars on the device: dev_state[0] scales lr (the schedule), dev_state[1] is the step
- * number t of the bias corrections 1 - beta^t.  Lets ONE captured CUDA graph of the whole training step (forward, backward,
- * gradient all-reduce, clip, AdamW) replay for every step: nothing the host passes changes between replays. */
+ * number t of the bias corrections 1 - beta^t, i.e. the count of APPLIED updates: the caller advances it after dadd_clip_coef
+ * only when coef[0] is finite (a skipped step does not count, as under torch.amp.GradScaler).  Lets ONE captured CUDA graph of
+ * the whole training step (forward, backward, gradient all-reduce, clip, AdamW) replay for every step: nothing the host passes
+ * changes between replays. */
 int dadd_adamw_step_dev(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2, float eps,
                         float weight_decay, const float* dev_state /* {lr scale, step} */, const float* coef, void* stream);
 /* EMA weight averaging of a flat fp32 parameter bucket: avg += (p - avg) * (1 - decay); first != 0: avg = p.  Replaces the

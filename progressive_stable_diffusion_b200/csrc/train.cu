@@ -408,14 +408,24 @@ __global__ void sum_small_kernel(const float* __restrict__ part, float* __restri
 // ------------------------------------------------------------------------------------------------ clipping + AdamW
 __global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g, int64_t n, float* __restrict__ part) {
     __shared__ float red[8];
+    // a thread's fp32 chain is folded into a double every 256 float4s: thousands of terms in one fp32 accumulator (few partials
+    // for a large buffer) drift low by a few 1e-6; shorter chains (every trainer bucket) give the plain fp32 sum, bit for bit
     float a = 0.0f;
+    double folded = 0.0;
+    int chain = 0;
     const int64_t n4 = n >> 2;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
         const float4 v = reinterpret_cast<const float4*>(g)[i];
         a = fmaf(v.x, v.x, fmaf(v.y, v.y, fmaf(v.z, v.z, fmaf(v.w, v.w, a))));
+        if (++chain == 256) {
+            folded += (double)a;
+            a = 0.0f;
+            chain = 0;
+        }
     }
     if (blockIdx.x == 0 && threadIdx.x == 0)
         for (int64_t i = n4 << 2; i < n; ++i) a = fmaf(g[i], g[i], a);
+    a = (float)(folded + (double)a);
     a = warp_sum(a);
     if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = a;
     __syncthreads();
@@ -599,7 +609,8 @@ extern "C" int dadd_minsnr_mse(const float* pred, const float* target, const flo
 extern "C" int64_t dadd_minsnr_mse_workspace_bytes(int B) { return (int64_t)B * 64 * sizeof(float); }
 
 extern "C" int dadd_sumsq(const float* g, int64_t n, float* partials, int n_partials, void* stream) {
-    DADD_REQUIRE(g && partials && n >= 0 && n_partials > 0 && ((uintptr_t)g % 16) == 0, "dadd_sumsq");
+    // (an empty buffer may come without an address: torch hands out NULL for zero elements; its partial sums are zeros)
+    DADD_REQUIRE((g || n == 0) && partials && n >= 0 && n_partials > 0 && ((uintptr_t)g % 16) == 0, "dadd_sumsq");
     sumsq_kernel<<<n_partials, 256, 0, (cudaStream_t)stream>>>(g, n, partials);
     return launched("dadd_sumsq");
 }

@@ -441,6 +441,8 @@ class DataParallelTrainer:
         # fp16 compute needs a loss scale (Lightning "16-mixed" runs a GradScaler): the backward pass sees loss * loss_scale, the
         # clip coefficient folds 1 / loss_scale back in, and a step whose scaled gradients overflowed is skipped on the device
         # (``step_overflowed`` reads the flag; halve ``loss_scale`` then).  bf16 (the default compute dtype) runs at 1.
+        # Like GradScaler.step, a skipped step leaves parameters and moments alone and does not advance AdamW's step count t
+        # (``optimizer_steps``); ``steps`` counts every step, as Lightning's global_step does, and keys the EMA schedule.
         self.loss_scale = float(loss_scale)
         self.betas, self.eps, self.weight_decay, self.max_grad_norm = betas, eps, weight_decay, max_grad_norm
         self.world = dist.get_world_size(process_group) if dist.is_initialized() else 1
@@ -478,6 +480,7 @@ class DataParallelTrainer:
         self.coef = torch.ones(2, device=dev, dtype=torch.float32)
         self.partials = torch.zeros(len(self.buckets), ops.SUMSQ_PARTIALS, device=dev, dtype=torch.float32)
         self.lr_scale = 1.0
+        self._torch_steps = 0                    # AdamW's t on the optimizer="torch" path
         # {lr scale, step number} as the fused AdamW reads them: on the device, advanced in stream order, so that a captured graph
         # of the whole step (``capture``) replays with the right schedule and bias corrections
         self.dev_state = torch.tensor([1.0, 0.0], device=dev, dtype=torch.float32) if dev.type == "cuda" else None
@@ -536,10 +539,11 @@ class DataParallelTrainer:
         b1, b2 = self.betas
         inv_world = 1.0 / (self.world * self.loss_scale)
         if self.optimizer == "fused":
-            self.dev_state[1:2].add_(1.0)                                   # the step number, in stream order (captured with the step)
             for i, bk in enumerate(self.buckets):
                 ops.sumsq_(bk.flat_g, self.partials[i])
             ops.clip_coef_(self.partials.view(-1), self.max_grad_norm, inv_world, self.coef)
+            # the step number, in stream order (captured with the step): advanced only when the update will be applied
+            self.dev_state[1:2].add_(torch.isfinite(self.coef[:1]))
             for bk in self.buckets:
                 if bk.m is None:
                     bk.m, bk.v = torch.zeros_like(bk.flat_p), torch.zeros_like(bk.flat_p)
@@ -547,18 +551,24 @@ class DataParallelTrainer:
                                     self.coef)
         else:       # reference arithmetic with stock PyTorch (CPU / gloo tests of the bucket logic)
             total = torch.sqrt(sum((bk.flat_g * inv_world).pow(2).sum() for bk in self.buckets))
+            applied = bool(torch.isfinite(total))         # the fused path's rule: a non-finite norm skips the step
             coef = inv_world * (torch.clamp(self.max_grad_norm / (total + 1e-6), max=1.0) if self.max_grad_norm > 0 else 1.0)
-            self.coef = torch.stack([torch.as_tensor(coef, dtype=torch.float32), total.float()])
+            self.coef = torch.stack([torch.as_tensor(coef if applied else math.nan, dtype=torch.float32, device=total.device),
+                                     total.float()])
             for bk in self.buckets:
                 if bk.m is None:
                     bk.m, bk.v = torch.zeros_like(bk.flat_p), torch.zeros_like(bk.flat_p)
-                g = bk.flat_g * coef
-                lr = bk.lr * self.lr_scale
-                bk.flat_p.mul_(1.0 - lr * self.weight_decay)
-                bk.m.mul_(b1).add_(g, alpha=1.0 - b1)
-                bk.v.mul_(b2).addcmul_(g, g, value=1.0 - b2)
-                denom = (bk.v.sqrt() / math.sqrt(1.0 - b2 ** self.steps)).add_(self.eps)
-                bk.flat_p.addcdiv_(bk.m, denom, value=-lr / (1.0 - b1 ** self.steps))
+            if applied:
+                self._torch_steps += 1
+                t = self._torch_steps
+                for bk in self.buckets:
+                    g = bk.flat_g * coef
+                    lr = bk.lr * self.lr_scale
+                    bk.flat_p.mul_(1.0 - lr * self.weight_decay)
+                    bk.m.mul_(b1).add_(g, alpha=1.0 - b1)
+                    bk.v.mul_(b2).addcmul_(g, g, value=1.0 - b2)
+                    denom = (bk.v.sqrt() / math.sqrt(1.0 - b2 ** t)).add_(self.eps)
+                    bk.flat_p.addcdiv_(bk.m, denom, value=-lr / (1.0 - b1 ** t))
         wcache.clear()        # inference-time derived weights (16-bit / fused copies) are stale after an in-place update
         if self.ema_decay is not None and self.ema_should_update(self.steps - 1):
             self.ema_update()
@@ -616,11 +626,13 @@ class DataParallelTrainer:
         """The dictionary Lightning + the EMA callback write (ema_callback.py:291-330): ``state_dict`` = averaged weights (what
         ``load_from_checkpoint`` and the inference / evaluation pipelines read), ``current_model_state`` = the weights training
         continues from, ``averaging_state`` = AveragedModel's own entries (``n_averaged``), the callback's ``latest_update_step``
-        and the optimizer moments per bucket (bucket order: resume with the same ``bucket_bytes`` / parameter groups).  Without
-        EMA: ``state_dict`` = the current weights."""
+        and the optimizer moments per bucket (bucket order: resume with the same ``bucket_bytes`` / parameter groups) with AdamW's
+        step count (``optimizer_step``: below ``global_step`` once a step has been skipped).  Without EMA: ``state_dict`` = the
+        current weights."""
         cur = {k: v.detach().clone() for k, v in self.module.state_dict().items()}
         ck = {"epoch": int(epoch), "global_step": int(self.steps), "state_dict": cur,
-              "optimizer_moments": [None if bk.m is None else (bk.m.clone(), bk.v.clone()) for bk in self.buckets]}
+              "optimizer_moments": [None if bk.m is None else (bk.m.clone(), bk.v.clone()) for bk in self.buckets],
+              "optimizer_step": self.optimizer_steps}
         if self.ema_decay is not None:
             ck["state_dict"] = self.ema_state_dict()
             ck["current_model_state"] = cur
@@ -630,12 +642,14 @@ class DataParallelTrainer:
 
     def load_checkpoint(self, ck: Dict) -> None:
         """Resume: the module takes ``current_model_state`` and the averages come from ``state_dict`` (on_load_checkpoint,
-        ema_callback.py:332-378); a checkpoint written without EMA initialises both from ``state_dict``."""
+        ema_callback.py:332-378); a checkpoint written without EMA initialises both from ``state_dict``.  A checkpoint without
+        ``optimizer_step`` (written before skipped steps were told apart) resumes AdamW's step count from ``global_step``."""
         names = {id(p): n for n, p in self.module.named_parameters()}
         self.module.load_state_dict(ck.get("current_model_state", ck["state_dict"]), strict=False)     # copies into the bucket views
         self.steps = int(ck.get("global_step", 0))
+        self._torch_steps = int(ck.get("optimizer_step", self.steps))
         if self.dev_state is not None:
-            self.dev_state[1:2].fill_(float(self.steps))
+            self.dev_state[1:2].fill_(float(self._torch_steps))
         if self.ema_decay is not None:
             for bk in self.buckets:
                 for p, off in zip(bk.params, bk.offsets):
@@ -750,6 +764,12 @@ class DataParallelTrainer:
     @property
     def grad_norm(self) -> torch.Tensor:
         return self.coef[1]
+
+    @property
+    def optimizer_steps(self) -> int:
+        """AdamW's step count t (``state["step"]`` of torch.optim.AdamW): the updates applied, skipped steps excluded.  The fused
+        optimizer keeps it on the device: reading it synchronises."""
+        return int(self.dev_state[1].item()) if self.optimizer == "fused" else self._torch_steps
 
     def step_overflowed(self) -> bool:
         """True when the last step was skipped because its (loss-scaled) gradients were not finite.  Synchronises."""

@@ -84,6 +84,8 @@ def test_argument_validation_of_the_newer_entry_points(lib):
     assert l.dadd_ema_update(16, 16, 64, 1.5, 0, None) != 0 and "decay" in err()
     assert l.dadd_ema_update(16, 24, 64, 0.9, 0, None) != 0                                           # 16-byte alignment
     assert l.dadd_adamw_step_dev(16, 16, 16, 16, 64, 1e-4, 0.9, 0.999, 1e-8, 0.01, None, None, None) != 0 and "dev_state" in err()
+    assert l.dadd_sumsq(None, 64, 16, 1, None) != 0 and "n == 0" in err()      # only an empty buffer may come without an address
+    assert l.dadd_sumsq(24, 64, 16, 1, None) != 0 and "dadd_sumsq" in err()    # 16-byte alignment
     assert l.dadd_groupnorm_cat_supported(4, 640, 320, 1024, 32, 1) == 1
     assert l.dadd_groupnorm_cat_supported(4, 644, 320, 1024, 32, 1) == 0    # C1 % 8
     assert l.dadd_groupnorm_cat_supported(4, 640, 320, 1024, 32, 0) == 0    # fp32

@@ -161,6 +161,87 @@ def test_checkpoint_layout_and_resume(tmp_path):
     assert all(torch.equal(e1[k], e2[k]) for k in e1)
 
 
+def _optimizer_state(tr):
+    """(p, m, v) of every bucket, cloned; moments not yet allocated read as zeros."""
+    zero = lambda bk: torch.zeros_like(bk.flat_p)
+    return [(bk.flat_p.clone(), zero(bk) if bk.m is None else bk.m.clone(), zero(bk) if bk.v is None else bk.v.clone())
+            for bk in tr.buckets]
+
+
+@pytest.mark.parametrize("overflow_at", [1, 3])
+def test_torch_optimizer_skips_overflowed_steps_like_grad_scaler(overflow_at):
+    """optimizer="torch" against Lightning's "16-mixed" step with gradient clipping (GradScaler: scale, backward, unscale_,
+    clip_grad_norm_, step, update) when the loss of one step is inf: that step leaves parameters and moments untouched, AdamW's
+    step count does not advance (GradScaler skips optimizer.step()), the caller halves the loss scale as the scaler does."""
+    torch.manual_seed(4)
+    m, ref = _Tiny(), _Tiny()
+    ref.load_state_dict(m.state_dict())
+    scale = 2.0 ** 13
+    tr = T.DataParallelTrainer(m, lr=1e-2, weight_decay=0.05, max_grad_norm=0.5, optimizer="torch", bucket_bytes=64, loss_scale=scale)
+    used = [p for n, p in ref.named_parameters() if n not in T.UNUSED_PARAMETERS]
+    groups = [{"params": [p for p in g["params"] if any(p is q for q in used)], "lr": g["lr"]} for g in T.parameter_groups(ref, 1e-2)]
+    opt = torch.optim.AdamW(groups, weight_decay=0.05)
+    scaler = torch.amp.GradScaler("cpu", init_scale=scale, growth_interval=10 ** 9)
+    x, y = torch.randn(16, 6), torch.randn(16, 4)
+    for s in range(1, 6):
+        flag = math.inf if s == overflow_at else 1.0
+        before = _optimizer_state(tr)
+        tr.step(lambda: ((m(x) - y) ** 2).mean() * flag)
+        opt.zero_grad()
+        scaler.scale(((ref(x) - y) ** 2).mean() * flag).backward()
+        scaler.unscale_(opt)
+        torch.nn.utils.clip_grad_norm_(used, 0.5)
+        scaler.step(opt)
+        scaler.update()
+        assert tr.step_overflowed() == (s == overflow_at), s
+        if tr.step_overflowed():
+            tr.loss_scale *= 0.5
+            for (p0, m0, v0), (p1, m1, v1) in zip(before, _optimizer_state(tr)):
+                assert torch.equal(p0, p1) and torch.equal(m0, m1) and torch.equal(v0, v1), s
+        assert tr.loss_scale == scaler.get_scale()
+        assert tr.steps == s and tr.optimizer_steps == s - (s >= overflow_at)
+        if s > overflow_at or overflow_at > 1:
+            assert int(opt.state[used[0]]["step"]) == tr.optimizer_steps
+        for (n, p), (_, q) in zip(m.named_parameters(), ref.named_parameters()):
+            torch.testing.assert_close(p, q, rtol=2e-5, atol=2e-6, msg=f"step {s}: {n}")
+
+
+def test_skipped_step_is_not_counted_by_adamw_and_survives_resume(tmp_path):
+    """global_step counts every step, AdamW's t the applied ones; the checkpoint keeps both, and a trainer resumed after a skipped
+    step continues bit for bit.  A checkpoint without ``optimizer_step`` resumes t from global_step."""
+    torch.manual_seed(5)
+    x, y = torch.randn(16, 6), torch.randn(16, 4)
+    kw = dict(lr=1e-2, weight_decay=0.05, max_grad_norm=0.5, optimizer="torch", bucket_bytes=64, ema_decay=0.9,
+              ema_update_every_n_steps=1, ema_update_starting_at_step=0)
+    m = _Tiny()
+    tr = T.DataParallelTrainer(m, **kw)
+    for flag in (1.0, math.inf):
+        tr.step(lambda: ((m(x) - y) ** 2).mean() * flag)
+    assert tr.step_overflowed() and tr.steps == 2 and tr.optimizer_steps == 1
+    assert all(torch.isfinite(p).all() for p in m.parameters())
+    path = tmp_path / "skipped.ckpt"
+    torch.save(tr.checkpoint(epoch=0), path)
+    ck = torch.load(path, weights_only=False)
+    assert ck["global_step"] == 2 and ck["optimizer_step"] == 1
+    m2 = _Tiny()
+    tr2 = T.DataParallelTrainer(m2, **kw)
+    tr2.load_checkpoint(ck)
+    assert tr2.steps == 2 and tr2.optimizer_steps == 1
+    for _ in range(3):
+        l1 = tr.step(lambda: ((m(x) - y) ** 2).mean())
+        l2 = tr2.step(lambda: ((m2(x) - y) ** 2).mean())
+        assert torch.equal(l1, l2)
+    assert tr2.optimizer_steps == tr.optimizer_steps == 4
+    for (n, p), (_, q) in zip(m.named_parameters(), m2.named_parameters()):
+        assert torch.equal(p, q), n
+    e1, e2 = tr.ema_state_dict(), tr2.ema_state_dict()
+    assert all(torch.equal(e1[k], e2[k]) for k in e1)
+    legacy = {k: v for k, v in ck.items() if k != "optimizer_step"}
+    tr3 = T.DataParallelTrainer(_Tiny(), **kw)
+    tr3.load_checkpoint(legacy)
+    assert tr3.optimizer_steps == 2
+
+
 def test_conditioning_train_functions_match_oracle():
     """aoe_train / purifier_train are the autograd twins of the inference kernels: same numbers as the (reference-pinned) oracle."""
     from progressive_stable_diffusion_b200.feature_purifier import FeaturePurifier
