@@ -30,7 +30,7 @@ extern "C" {
 
 /* ABI version of this header (bumped on any signature change).  The host binding refuses a library whose
  * dadd_abi_version() differs from the DADD_ABI_VERSION it was written against. */
-#define DADD_ABI_VERSION 13
+#define DADD_ABI_VERSION 14
 int dadd_abi_version(void);
 /* Message of the last failing call on this thread ("" if none). */
 const char* dadd_last_error(void);
@@ -274,6 +274,28 @@ int dadd_adamw_step_dev(float* p, const float* g, float* m, float* v, int64_t n,
  * AveragedModel.update_parameters call of the reference's EMAWeightAveraging callback (src/callbacks/ema_callback.py:168-197,414-436:
  * torch.optim.swa_utils.get_ema_avg_fn(decay), decay 0.999, every 4th step from step 100 in configs/train_ip.yaml:83-85). */
 int dadd_ema_update(float* avg, const float* p, int64_t n, float decay, int first, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Pairwise squared-distance statistics of two fp32 feature sets, for the CMMD and improved precision / recall metrics.
+ * Replaces the distance matrices of the evaluation metrics (src/pipelines/evaluation/evaluation_pipeline.py:577-839,978-1179:
+ * CMMD's `mmd` of google-research/cmmd and the k-NN radii / coverage of Kynkaanniemi et al. 2019), none of which is
+ * materialised here.  x: [M][D], y: [N][D], dense row-major fp32, 16-byte aligned;
+ *   d2[i][j] = max(|x_i|^2 + |y_j|^2 - 2 x_i . y_j, 0), the dot products by error-compensated TF32 (3 tcgen05 passes, fp32 accumulate).
+ * mode DADD_PAIRWISE_RBF_SUM: out = double[1] = sum over all (i, j) of exp(-gamma d2[i][j]) (fixed-order, atomics-free sums:
+ *      bit-reproducible);
+ *      DADD_PAIRWISE_KNN:     out = float[M], the k-th smallest d2[i][j] over j (1 <= k <= 16; N > k, or N > k + 1 with same_set);
+ *      DADD_PAIRWISE_COVER:   out = uint8[M], 1 where some j has d2[i][j] <= radii[j] (radii: float[N], required).
+ * same_set (RBF_SUM, KNN): y is x (pass y = NULL or x, N = M); KNN then excludes j == i by index.  D % 8 == 0.
+ * workspace: at least dadd_pairwise_workspace_bytes(...) bytes (-1: the arguments are rejected), 16-byte aligned: the tf32
+ * hi / lo split of the rows ((M + N) * D * 8 bytes, M * D * 8 with same_set), the row norms and the per-slice partials (RBF_SUM:
+ * one double per (128-row block, column slice); KNN: M * slices * k floats; COVER: M * slices bytes); never an M x N buffer. */
+#define DADD_PAIRWISE_RBF_SUM 0
+#define DADD_PAIRWISE_KNN 1
+#define DADD_PAIRWISE_COVER 2
+int64_t dadd_pairwise_workspace_bytes(int64_t M, int64_t N, int D, int mode, int k, int same_set);
+int dadd_pairwise(const float* x, const float* y /* NULL or x with same_set */, int64_t M, int64_t N, int D, int mode, int k,
+                  int same_set, float gamma, const float* radii /* COVER only */, void* out, void* workspace,
+                  int64_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

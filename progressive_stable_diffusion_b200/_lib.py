@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("DADD_B200_LIB") or os.path.join(HERE, "libdadd_b200.s
 
 _P, _I, _L, _F = c_void_p, c_int, c_int64, c_float
 
-ABI_VERSION = 13         # == DADD_ABI_VERSION of include/dadd_b200.h that SIGNATURES below was written against
+ABI_VERSION = 14         # == DADD_ABI_VERSION of include/dadd_b200.h that SIGNATURES below was written against
 
 # name -> argtypes; mirrors include/dadd_b200.h one to one (tests/test_abi.py checks header <-> table <-> .so)
 SIGNATURES = {
@@ -56,6 +56,9 @@ SIGNATURES = {
     "dadd_adamw_step": [_P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _F, _F, _P, _P],
     "dadd_adamw_step_dev": [_P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _P, _P, _P],
     "dadd_ema_update": [_P, _P, _L, _F, _I, _P],
+    # evaluation metrics
+    "dadd_pairwise_workspace_bytes": [_L, _L, _I, _I, _I, _I],
+    "dadd_pairwise": [_P, _P, _L, _L, _I, _I, _I, _I, _F, _P, _P, _P, _L, _P],
 }
 
 _lib = None

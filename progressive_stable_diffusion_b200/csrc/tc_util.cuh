@@ -78,6 +78,18 @@ __device__ __forceinline__ void mma_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_
         ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(acc)
         : "memory");
 }
+// kind::tf32: fp32 operands in shared memory (the tensor core reads the top 19 bits of each), fp32 accumulate, M = 128.
+// Same descriptor layout as kind::f16 with format code 2 (cute::UMMA::F16F32Format::TF32); one MMA covers K = 8 (32 bytes).
+__host__ __device__ constexpr uint32_t instr_desc_tf32(uint32_t n) { return instr_desc(2u, n, 0u); }
+
+__device__ __forceinline__ void mma_ss_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(acc)
+        : "memory");
+}
+
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }

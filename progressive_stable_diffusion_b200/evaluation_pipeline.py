@@ -1,8 +1,9 @@
 """Batched evaluation sampling for B200: the sampling half of
 ``/root/reference/src/pipelines/evaluation/evaluation_pipeline.py`` (``_prepare_conditioning`` :406-461,
 ``_set_delta_scale`` :464-468, ``_ddim_sample_batched`` :471-564, ``_decode_latents`` :567-574, ``GenerationJob`` / ``_collect_jobs``
-:83-89,843-864, the job order, batching and per-class grouping of ``generate_all`` :867-975).  The FID / CMMD / P&R metrics of that file use third-party backbones and are not on the
-denoising path (SURVEY.md section 2, row 9).
+:83-89,843-864, the job order, batching and per-class grouping of ``generate_all`` :867-975) - and its scoring: ``evaluate_images`` computes CMMD and improved precision / recall per target class
+(``evaluate_one_run`` :577-839,978-1179) on ``metrics.py``.  A sweep runs ``generate_all`` -> ``group_by_target`` ->
+``evaluate_images``.  FID is not computed: its backbone, torch-fidelity's TF-ported InceptionV3, is not available here.
 """
 
 from __future__ import annotations
@@ -14,7 +15,7 @@ from typing import Dict, List, Optional, Sequence, Tuple
 import torch
 from torch import Tensor
 
-from . import parallel
+from . import metrics, parallel
 from .inference_pipeline_ip import (_latents_to_images, _prepare_conditioning as _prep, _sample,
                                     _set_delta_scale_on_processors)
 
@@ -141,4 +142,29 @@ def generate_all(module, jobs: Sequence[Tuple[int, float, float]], image_tokens:
         res = _decode_latents(module, lat) if decode else lat.cpu()
         for k, i in enumerate(idx):
             out[i] = res[k]
+    return out
+
+
+@torch.no_grad()
+def evaluate_images(real_by_class: Dict[int, Tensor], fake_by_class: Dict[int, Tensor], clip: "metrics.ClipEmbedder",
+                    vgg: "metrics.VGGFeatures", k: int = 3) -> Dict[object, Dict[str, float]]:
+    """CMMD and improved precision / recall of generated against real [0, 1] images, per target class and over all classes.
+    ``real_by_class`` / ``fake_by_class``: ``{class: (N, 3, H, W)}`` as ``group_by_target`` returns them.  Returns
+    ``{class: {"cmmd", "precision", "recall"}, ..., "all": {...}}``.  A class missing or empty on either side is left out;
+    precision and recall are NaN where a side has k + 1 points or fewer (a k-NN radius needs k other points and more)."""
+    out: Dict[object, Dict[str, float]] = {}
+    feats = {}
+    for cls in ALL_MES_CLASSES:
+        real, fake = real_by_class.get(cls), fake_by_class.get(cls)
+        if real is None or fake is None or real.shape[0] == 0 or fake.shape[0] == 0:
+            continue
+        feats[cls] = (clip(real), clip(fake), vgg(real), vgg(fake))
+    groups = list(feats.items())
+    if feats:
+        groups.append(("all", tuple(torch.cat([f[i] for f in feats.values()]) for i in range(4))))
+    for key, (cr, cf, vr, vf) in groups:
+        res = {"cmmd": metrics.cmmd(cr, cf), "precision": float("nan"), "recall": float("nan")}
+        if min(vr.shape[0], vf.shape[0]) > k + 1:
+            res["precision"], res["recall"] = metrics.precision_recall(vr, vf, k)
+        out[key] = res
     return out

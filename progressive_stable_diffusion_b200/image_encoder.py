@@ -26,6 +26,7 @@ from .attention_processor import compute_dtype
 
 _ARCH = {   # pretrained_path suffix -> (hidden, intermediate, layers, heads, image, patch, projection)
     "clip-vit-large-patch14": (1024, 4096, 24, 16, 224, 14, 768),
+    "clip-vit-large-patch14-336": (1024, 4096, 24, 16, 336, 14, 768),      # CMMD's embedding (metrics.ClipEmbedder)
     "clip-vit-base-patch16": (768, 3072, 12, 12, 224, 16, 512),
     "clip-vit-base-patch32": (768, 3072, 12, 12, 224, 32, 512),
 }

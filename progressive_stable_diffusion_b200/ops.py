@@ -509,3 +509,54 @@ def adamw_step_(p: torch.Tensor, g: torch.Tensor, m: torch.Tensor, v: torch.Tens
     _lib.check(_lib.load().dadd_adamw_step(p.data_ptr(), g.data_ptr(), m.data_ptr(), v.data_ptr(), p.numel(), lr, beta1, beta2, eps,
                                            weight_decay, 1.0 - beta1 ** step, 1.0 - beta2 ** step, _ptr(coef), _stream()),
                "dadd_adamw_step")
+
+
+# --------------------------------------------------------------------------------------------- evaluation metrics
+RBF_SUM, KNN, COVER = 0, 1, 2
+
+
+def _features(*ts: torch.Tensor) -> None:
+    _cuda(*ts)
+    for t in ts:
+        if t.dtype != torch.float32 or t.dim() != 2 or not t.is_contiguous():
+            raise _lib.DaddError(f"pairwise statistics take contiguous 2-D float32 feature matrices, got {t.dtype} {tuple(t.shape)}")
+
+
+def _pairwise(x: torch.Tensor, y: Optional[torch.Tensor], mode: int, out: torch.Tensor, k: int = 0, gamma: float = 0.0,
+              radii: Optional[torch.Tensor] = None) -> torch.Tensor:
+    lib = _lib.load()
+    m, d = x.shape
+    n = m if y is None else y.shape[0]
+    if y is not None and y.shape[1] != d:
+        raise _lib.DaddError(f"feature widths differ: {d} vs {y.shape[1]}")
+    same = int(y is None)
+    ws_bytes = int(lib.dadd_pairwise_workspace_bytes(m, n, d, mode, k, same))
+    if ws_bytes < 0:
+        _lib.check(1, "dadd_pairwise_workspace_bytes")
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+    _lib.check(lib.dadd_pairwise(x.data_ptr(), _ptr(y), m, n, d, mode, k, same, float(gamma), _ptr(radii), out.data_ptr(),
+                                 ws.data_ptr(), ws_bytes, _stream()), "dadd_pairwise")
+    return out
+
+
+def pairwise_rbf_sum(x: torch.Tensor, y: Optional[torch.Tensor], gamma: float) -> torch.Tensor:
+    """sum over all (i, j) of exp(-gamma |x_i - y_j|^2) as a float64 device scalar; ``y=None``: y is x.  x: (M, D), y: (N, D)
+    float32, D % 8 == 0 (the kernel sums of google-research/cmmd's ``mmd``)."""
+    _features(x, *(() if y is None else (y,)))
+    return _pairwise(x, y, RBF_SUM, torch.empty((), dtype=torch.float64, device=x.device), gamma=gamma)
+
+
+def knn_radii(x: torch.Tensor, k: int) -> torch.Tensor:
+    """(M,) float32: the squared distance from each row of x to its k-th nearest OTHER row (1 <= k <= 16, M > k + 1): the
+    manifold radii of improved precision / recall (Kynkaanniemi et al. 2019)."""
+    _features(x)
+    return _pairwise(x, None, KNN, torch.empty(x.shape[0], dtype=torch.float32, device=x.device), k=k)
+
+
+def within_radii(q: torch.Tensor, ref: torch.Tensor, radii: torch.Tensor) -> torch.Tensor:
+    """(M,) bool: whether each row of q lies in at least one ball |q_i - ref_j|^2 <= radii[j] (improved precision / recall)."""
+    _features(q, ref)
+    _cuda(radii)
+    if radii.dtype != torch.float32 or radii.shape != (ref.shape[0],) or not radii.is_contiguous():
+        raise _lib.DaddError(f"radii must be a contiguous float32 ({ref.shape[0]},) tensor")
+    return _pairwise(q, ref, COVER, torch.empty(q.shape[0], dtype=torch.bool, device=q.device), radii=radii)
