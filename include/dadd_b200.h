@@ -30,7 +30,7 @@ extern "C" {
 
 /* ABI version of this header (bumped on any signature change).  The host binding refuses a library whose
  * dadd_abi_version() differs from the DADD_ABI_VERSION it was written against. */
-#define DADD_ABI_VERSION 14
+#define DADD_ABI_VERSION 15
 int dadd_abi_version(void);
 /* Message of the last failing call on this thread ("" if none). */
 const char* dadd_last_error(void);
@@ -276,7 +276,8 @@ int dadd_adamw_step_dev(float* p, const float* g, float* m, float* v, int64_t n,
 int dadd_ema_update(float* avg, const float* p, int64_t n, float decay, int first, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
- * Pairwise squared-distance statistics of two fp32 feature sets, for the CMMD and improved precision / recall metrics.
+ * Pairwise squared-distance statistics of two fp32 feature sets, for the CMMD, improved precision / recall, density / coverage
+ * and realism metrics.
  * Replaces the distance matrices of the evaluation metrics (src/pipelines/evaluation/evaluation_pipeline.py:577-839,978-1179:
  * CMMD's `mmd` of google-research/cmmd and the k-NN radii / coverage of Kynkaanniemi et al. 2019), none of which is
  * materialised here.  x: [M][D], y: [N][D], dense row-major fp32, 16-byte aligned;
@@ -284,17 +285,26 @@ int dadd_ema_update(float* avg, const float* p, int64_t n, float decay, int firs
  * mode DADD_PAIRWISE_RBF_SUM: out = double[1] = sum over all (i, j) of exp(-gamma d2[i][j]) (fixed-order, atomics-free sums:
  *      bit-reproducible);
  *      DADD_PAIRWISE_KNN:     out = float[M], the k-th smallest d2[i][j] over j (1 <= k <= 16; N > k, or N > k + 1 with same_set);
- *      DADD_PAIRWISE_COVER:   out = uint8[M], 1 where some j has d2[i][j] <= radii[j] (radii: float[N], required).
+ *      DADD_PAIRWISE_COVER:   out = uint8[M], 1 where some j has d2[i][j] <= radii[j];
+ *      DADD_PAIRWISE_COUNT:   out = int32[M], the number of j with d2[i][j] <= radii[j];
+ *      DADD_PAIRWISE_RATIO_MAX: out = float[M], the max over j of radii[j] / (d2[i][j] + eps) (IEEE fp32 division, 0 when no
+ *                             ratio is positive), eps passed in `gamma`: finite and > 0.
+ * COVER, COUNT and RATIO_MAX need radii (float[N]) and reject same_set.  Counts, flags and maxima are merged in a fixed order:
+ * every mode is bit-reproducible and independent of the grid.
  * same_set (RBF_SUM, KNN): y is x (pass y = NULL or x, N = M); KNN then excludes j == i by index.  D % 8 == 0.
  * workspace: at least dadd_pairwise_workspace_bytes(...) bytes (-1: the arguments are rejected), 16-byte aligned: the tf32
  * hi / lo split of the rows ((M + N) * D * 8 bytes, M * D * 8 with same_set), the row norms and the per-slice partials (RBF_SUM:
- * one double per (128-row block, column slice); KNN: M * slices * k floats; COVER: M * slices bytes); never an M x N buffer. */
+ * one double per (128-row block, column slice); KNN: M * slices * k floats; COVER, COUNT: M * slices int32 counts; RATIO_MAX:
+ * M * slices floats); never an M x N buffer. */
 #define DADD_PAIRWISE_RBF_SUM 0
 #define DADD_PAIRWISE_KNN 1
 #define DADD_PAIRWISE_COVER 2
+#define DADD_PAIRWISE_COUNT 3
+#define DADD_PAIRWISE_RATIO_MAX 4
 int64_t dadd_pairwise_workspace_bytes(int64_t M, int64_t N, int D, int mode, int k, int same_set);
 int dadd_pairwise(const float* x, const float* y /* NULL or x with same_set */, int64_t M, int64_t N, int D, int mode, int k,
-                  int same_set, float gamma, const float* radii /* COVER only */, void* out, void* workspace,
+                  int same_set, float gamma /* RBF_SUM: gamma; RATIO_MAX: eps */,
+                  const float* radii /* COVER, COUNT, RATIO_MAX */, void* out, void* workspace,
                   int64_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus

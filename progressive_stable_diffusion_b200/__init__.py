@@ -13,7 +13,7 @@ from .attention_processor_routing_gates import (SplitInjectionAttentionProcessor
 from .diffusion_module_ip import DiffusionIPConfig, DiffusionModuleWithIP, default_config, load_config  # noqa: F401
 from .feature_purifier import FeaturePurifier  # noqa: F401
 from .image_encoder import ImageEncoder, ImageProjection, ImageProjectionPlus  # noqa: F401
-from .metrics import ClipEmbedder, VGGFeatures, cmmd, precision_recall  # noqa: F401
+from .metrics import ClipEmbedder, VGGFeatures, cmmd, density_coverage, precision_recall, realism_scores  # noqa: F401
 from .ordinal_embedder import AdditiveOrdinalEmbedder  # noqa: F401
 from .unet import OrdinalUNet, UNetConfig  # noqa: F401
 from .vae import SDVAE  # noqa: F401
@@ -23,5 +23,5 @@ __all__ = [
     "get_frequency_mode_for_block", "set_ordinal_ip_attention_processors", "set_split_injection_processors",
     "DiffusionIPConfig", "DiffusionModuleWithIP", "default_config", "load_config", "FeaturePurifier",
     "AdditiveOrdinalEmbedder", "OrdinalUNet", "UNetConfig", "SDVAE", "ImageEncoder", "ImageProjection", "ImageProjectionPlus",
-    "ClipEmbedder", "VGGFeatures", "cmmd", "precision_recall",
+    "ClipEmbedder", "VGGFeatures", "cmmd", "precision_recall", "density_coverage", "realism_scores",
 ]

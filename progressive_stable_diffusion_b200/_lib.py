@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("DADD_B200_LIB") or os.path.join(HERE, "libdadd_b200.s
 
 _P, _I, _L, _F = c_void_p, c_int, c_int64, c_float
 
-ABI_VERSION = 14         # == DADD_ABI_VERSION of include/dadd_b200.h that SIGNATURES below was written against
+ABI_VERSION = 15         # == DADD_ABI_VERSION of include/dadd_b200.h that SIGNATURES below was written against
 
 # name -> argtypes; mirrors include/dadd_b200.h one to one (tests/test_abi.py checks header <-> table <-> .so)
 SIGNATURES = {

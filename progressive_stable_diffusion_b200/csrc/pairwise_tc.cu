@@ -1,12 +1,14 @@
-// Pairwise squared-distance statistics of two fp32 feature sets without the distance matrix: the CMMD and improved
-// precision / recall metrics of the evaluation sweep (reference: src/pipelines/evaluation/evaluation_pipeline.py:577-839,
-// 978-1179, which materialise cdist matrices in torch).
+// Pairwise squared-distance statistics of two fp32 feature sets without the distance matrix: the CMMD, improved precision /
+// recall, density / coverage and realism metrics of the evaluation sweep (reference: src/pipelines/evaluation/
+// evaluation_pipeline.py:577-839, 978-1179, which materialise cdist matrices in torch).
 //   d2[i][j] = max(|x_i|^2 + |y_j|^2 - 2 x_i . y_j, 0)       X: [M][D], Y: [N][D], row-major fp32
 // One persistent tcgen05 GEMM computes 128 x 256 tiles of X Y^T into TMEM; the epilogue turns each tile into d2 and folds
 // it into per-(row, column slice) state, so no distance ever reaches global memory:
 //   RBF_SUM  sum_ij exp(-gamma d2)         per-row sums in double, one partial per (row block, slice), summed in fixed order
 //   KNN      k-th smallest d2 of each row  per-slice sorted top-k lists, merged by a second pass (same_set: j == i excluded)
-//   COVER    exists j: d2[i][j] <= r[j]    per-slice flags, OR-merged
+//   COUNT    #{j : d2[i][j] <= r[j]}       per-slice int32 counts, summed; COVER is the same count, finished as count > 0
+//   RATIO_MAX max_j r[j] / (d2[i][j] + eps) per-slice maxima (IEEE division, running max from 0), max-merged
+// COVER, COUNT and RATIO_MAX share one kernel instance (the radius instance): Args::mode picks the reduction once per tile.
 // Precision: fp32-faithful via error-compensated TF32.  A pre-pass splits every row into hi = tf32(x) (round to nearest) and
 // lo = x - hi (exact in fp32) and computes |x|^2 in double; the MMA accumulates lo_x.hi_y + hi_x.lo_y + hi_x.hi_y (kind::tf32,
 // fp32 in TMEM).  What is dropped is lo_x.lo_y (<= 2^-22 |x||y|) and the tf32 truncation of lo (<= 2^-21 |x||y| per term).
@@ -61,7 +63,7 @@ static Plan make_plan(int64_t M, int64_t N, int D, int mode, int k, int same_set
     p.off_part = o;
     if (mode == DADD_PAIRWISE_RBF_SUM) o += up256(p.items * 8);
     else if (mode == DADD_PAIRWISE_KNN) o += up256(M * p.S * k * 4);
-    else o += up256(M * p.S);
+    else o += up256(M * p.S * 4);                 // radius modes: one int32 count or float max per (row, slice)
     p.total = o;
     return p;
 }
@@ -130,10 +132,30 @@ __global__ void __launch_bounds__(256) split_kernel(const float* __restrict__ x,
 struct Args {
     const float *nx, *ny, *radii;
     void* part;
-    int M, N, D, k, same_set;
-    float gamma;
+    int M, N, D, k, same_set, mode;
+    float gamma;                                  // RBF_SUM: gamma; RATIO_MAX: eps
     int S, tps, nct, items;
 };
+
+// The radius instance's reduction of one 128 x 256 TMEM tile into this thread's row: a count of d2 <= r (COUNT, COVER) or a
+// running max of r / (d2 + eps) (RATIO_MAX).  Padded columns have r = -1: they neither count nor raise the max (which starts at 0).
+template <bool RATIO>
+__device__ __forceinline__ void radius_tile(uint32_t taddr, const float* ny, const float* rr, float nxi, float eps, int& cnt,
+                                            float& rmax) {
+#pragma unroll 1
+    for (int ch = 0; ch < TBN / 32; ++ch) {
+        uint32_t v[32];
+        tmem_ld32(taddr + ch * 32, v);
+        tmem_wait_ld();
+#pragma unroll
+        for (int e = 0; e < 32; ++e) {
+            const int j = ch * 32 + e;
+            const float d2 = fmaxf(fmaf(-2.0f, __uint_as_float(v[e]), nxi + ny[j]), 0.0f);
+            if (RATIO) rmax = fmaxf(rmax, __fdiv_rn(rr[j], d2 + eps));
+            else cnt += d2 <= rr[j] ? 1 : 0;
+        }
+    }
+}
 
 template <int MODE>
 __global__ void __launch_bounds__(NTHREADS, 1)
@@ -146,7 +168,7 @@ pairwise_kernel(const __grid_constant__ CUtensorMap txh, const __grid_constant__
     unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     unsigned char* sStage = smem;
     float* sNy = reinterpret_cast<float*>(sStage + STAGES * STAGE_BYTES);     // [2 accumulators][TBN]
-    float* sR = sNy + 2 * TBN;                                                  // [2][TBN] (COVER)
+    float* sR = sNy + 2 * TBN;                                                  // [2][TBN] (radius modes)
     double* sRed = reinterpret_cast<double*>(sR + 2 * TBN);                     // [4] (RBF_SUM)
     Bars* bars = reinterpret_cast<Bars*>(sRed + 4);
 
@@ -242,7 +264,8 @@ pairwise_kernel(const __grid_constant__ CUtensorMap txh, const __grid_constant__
 #pragma unroll
             for (int q = 0; q < KMAX; ++q) best[q] = __int_as_float(0x7f800000);
             float kth = __int_as_float(0x7f800000);
-            bool cov = false;
+            int cnt = 0;
+            float rmax = 0.0f;
             const int ct_end = min(p.nct, (s + 1) * p.tps);
             for (int ct = s * p.tps; ct < ct_end; ++ct, ++t) {
                 const uint32_t a = t & 1;
@@ -252,29 +275,30 @@ pairwise_kernel(const __grid_constant__ CUtensorMap txh, const __grid_constant__
                 for (int j = row; j < TBN; j += 128) {                // (slot a was last read two tiles ago)
                     const int col = c0 + j;
                     ny[j] = col < p.N ? p.ny[col] : 0.0f;
-                    if (MODE == DADD_PAIRWISE_COVER) rr[j] = col < p.N ? p.radii[col] : -1.0f;
+                    if (MODE == DADD_PAIRWISE_COUNT) rr[j] = col < p.N ? p.radii[col] : -1.0f;
                 }
                 mbar_wait(&bars->acc_full[a], (t >> 1) & 1);
                 fence_after();
                 named_sync(1, 128);
+                if (MODE == DADD_PAIRWISE_COUNT) {
+                    if (p.mode == DADD_PAIRWISE_RATIO_MAX) radius_tile<true>(tmem + a * TBN + lane_base, ny, rr, nxi, p.gamma, cnt, rmax);
+                    else radius_tile<false>(tmem + a * TBN + lane_base, ny, rr, nxi, p.gamma, cnt, rmax);
+                } else {
 #pragma unroll 1
-                for (int ch = 0; ch < TBN / 32; ++ch) {
-                    uint32_t v[32];
-                    tmem_ld32(tmem + a * TBN + ch * 32 + lane_base, v);
-                    tmem_wait_ld();
+                    for (int ch = 0; ch < TBN / 32; ++ch) {
+                        uint32_t v[32];
+                        tmem_ld32(tmem + a * TBN + ch * 32 + lane_base, v);
+                        tmem_wait_ld();
 #pragma unroll
-                    for (int e = 0; e < 32; ++e) {
-                        const int j = ch * 32 + e, col = c0 + j;
-                        const float d2 = fmaxf(fmaf(-2.0f, __uint_as_float(v[e]), nxi + ny[j]), 0.0f);
-                        if (MODE == DADD_PAIRWISE_RBF_SUM) {
-                            if (col < p.N) rsum += (double)expf(-p.gamma * d2);
-                        } else if (MODE == DADD_PAIRWISE_KNN) {
-                            if (col < p.N && d2 < kth && !(p.same_set && col == gi)) {
+                        for (int e = 0; e < 32; ++e) {
+                            const int j = ch * 32 + e, col = c0 + j;
+                            const float d2 = fmaxf(fmaf(-2.0f, __uint_as_float(v[e]), nxi + ny[j]), 0.0f);
+                            if (MODE == DADD_PAIRWISE_RBF_SUM) {
+                                if (col < p.N) rsum += (double)expf(-p.gamma * d2);
+                            } else if (col < p.N && d2 < kth && !(p.same_set && col == gi)) {
                                 topk_insert(best, d2, p.k);
                                 kth = topk_last(best, p.k);
                             }
-                        } else {
-                            cov |= d2 <= rr[j];                       // (rr = -1 beyond N)
                         }
                     }
                 }
@@ -295,8 +319,10 @@ pairwise_kernel(const __grid_constant__ CUtensorMap txh, const __grid_constant__
 #pragma unroll
                     for (int q = 0; q < KMAX; ++q)
                         if (q < p.k) dst[q] = best[q];
+                } else if (p.mode == DADD_PAIRWISE_RATIO_MAX) {
+                    reinterpret_cast<float*>(p.part)[(int64_t)gi * p.S + s] = rmax;
                 } else {
-                    reinterpret_cast<uint8_t*>(p.part)[(int64_t)gi * p.S + s] = cov ? 1 : 0;
+                    reinterpret_cast<int*>(p.part)[(int64_t)gi * p.S + s] = cnt;
                 }
             }
         }
@@ -334,12 +360,22 @@ __global__ void knn_finish_kernel(const float* __restrict__ part, int M, int S, 
     out[i] = topk_last(best, k);
 }
 
-__global__ void cover_finish_kernel(const uint8_t* __restrict__ part, int M, int S, uint8_t* __restrict__ out) {
+// Radius modes, slices in order: COUNT sums the counts (int32 out), COVER writes count > 0 (uint8 out), RATIO_MAX takes the max.
+__global__ void radius_finish_kernel(const void* __restrict__ part, int M, int S, int mode, void* __restrict__ out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= M) return;
-    uint8_t f = 0;
-    for (int s = 0; s < S; ++s) f |= part[(int64_t)i * S + s];
-    out[i] = f;
+    if (mode == DADD_PAIRWISE_RATIO_MAX) {
+        const float* src = reinterpret_cast<const float*>(part) + (int64_t)i * S;
+        float r = 0.0f;
+        for (int s = 0; s < S; ++s) r = fmaxf(r, src[s]);
+        reinterpret_cast<float*>(out)[i] = r;
+        return;
+    }
+    const int* src = reinterpret_cast<const int*>(part) + (int64_t)i * S;
+    int c = 0;
+    for (int s = 0; s < S; ++s) c += src[s];
+    if (mode == DADD_PAIRWISE_COUNT) reinterpret_cast<int*>(out)[i] = c;
+    else reinterpret_cast<uint8_t*>(out)[i] = c > 0 ? 1 : 0;
 }
 
 // 2-D row-major fp32 (rows, cols), box = 32 columns (128 bytes) x box_rows, 128-byte swizzle, zero fill beyond the edges
@@ -372,13 +408,17 @@ static int launch_main(const CUtensorMap (&maps)[4], const Args& a, cudaStream_t
 
 using namespace daddk;
 
+static bool radius_mode(int mode) {
+    return mode == DADD_PAIRWISE_COVER || mode == DADD_PAIRWISE_COUNT || mode == DADD_PAIRWISE_RATIO_MAX;
+}
+
 static int pairwise_check(int64_t M, int64_t N, int D, int mode, int k, int same_set) {
-    if (mode != DADD_PAIRWISE_RBF_SUM && mode != DADD_PAIRWISE_KNN && mode != DADD_PAIRWISE_COVER)
+    if (mode != DADD_PAIRWISE_RBF_SUM && mode != DADD_PAIRWISE_KNN && !radius_mode(mode))
         return fail("%s: unknown mode %lld", "dadd_pairwise", (long long)mode);
     if (M < 1 || N < 1 || M > (1ll << 30) || N > (1ll << 30))
         return fail("%s: needs 1 <= M, N <= 2^30 (M = %lld, N = %lld)", "dadd_pairwise", (long long)M, (long long)N);
     if (D < 8 || D % 8 != 0 || D > (1 << 20)) return fail("%s: needs D %% 8 == 0 and 8 <= D <= 2^20 (D = %lld)", "dadd_pairwise", (long long)D);
-    if (same_set && (N != M || mode == DADD_PAIRWISE_COVER))
+    if (same_set && (N != M || radius_mode(mode)))
         return fail("%s: same_set needs N == M and mode RBF_SUM or KNN (N = %lld, M = %lld)", "dadd_pairwise", (long long)N, (long long)M);
     if (mode == DADD_PAIRWISE_KNN) {
         if (k < 1 || k > pw::KMAX) return fail("%s: KNN needs 1 <= k <= 16 (k = %lld)", "dadd_pairwise", (long long)k);
@@ -399,7 +439,9 @@ extern "C" int dadd_pairwise(const float* x, const float* y, int64_t M, int64_t 
     if (pairwise_check(M, N, D, mode, k, same_set)) return 1;
     DADD_REQUIRE(x && out && workspace, "dadd_pairwise");
     DADD_REQUIRE(same_set ? (y == nullptr || y == x) : y != nullptr, "dadd_pairwise");
-    if (mode == DADD_PAIRWISE_COVER && !radii) return fail("%s: COVER needs radii (got NULL)", "dadd_pairwise");
+    if (radius_mode(mode) && !radii) return fail("%s: COVER, COUNT and RATIO_MAX need radii (got NULL)", "dadd_pairwise");
+    if (mode == DADD_PAIRWISE_RATIO_MAX && !(gamma > 0.0f && gamma < INFINITY))
+        return fail("%s: RATIO_MAX needs a finite eps > 0, passed as gamma (eps = %g)", "dadd_pairwise", (double)gamma);
     DADD_REQUIRE(((uintptr_t)x | (uintptr_t)y | (uintptr_t)workspace) % 16 == 0, "dadd_pairwise");
     const pw::Plan pl = pw::make_plan(M, N, D, mode, k, same_set);
     if (workspace_bytes < pl.total)
@@ -419,15 +461,16 @@ extern "C" int dadd_pairwise(const float* x, const float* y, int64_t M, int64_t 
         pw::split_kernel<<<(unsigned)((N + 7) / 8), 256, 0, s>>>(y, yhi, ylo, ny, N, D);
         if (int rc = launched("dadd_pairwise split")) return rc;
     }
-    pw::Args a{nx, ny, radii, ws + pl.off_part, (int)M, (int)N, D, k, same_set, gamma, (int)pl.S, (int)pl.tps, (int)pl.nct, (int)pl.items};
+    pw::Args a{nx, ny, radii, ws + pl.off_part, (int)M, (int)N, D, k, same_set, mode, gamma, (int)pl.S, (int)pl.tps, (int)pl.nct,
+               (int)pl.items};
     int rc;
     if (mode == DADD_PAIRWISE_RBF_SUM) rc = pw::launch_main<DADD_PAIRWISE_RBF_SUM>(maps, a, s);
     else if (mode == DADD_PAIRWISE_KNN) rc = pw::launch_main<DADD_PAIRWISE_KNN>(maps, a, s);
-    else rc = pw::launch_main<DADD_PAIRWISE_COVER>(maps, a, s);
+    else rc = pw::launch_main<DADD_PAIRWISE_COUNT>(maps, a, s);     // the radius instance: COVER, COUNT, RATIO_MAX
     if (rc) return rc;
     const unsigned fb = (unsigned)((M + 255) / 256);
     if (mode == DADD_PAIRWISE_RBF_SUM) pw::rbf_finish_kernel<<<1, 1024, 0, s>>>((const double*)a.part, a.items, (double*)out);
     else if (mode == DADD_PAIRWISE_KNN) pw::knn_finish_kernel<<<fb, 256, 0, s>>>((const float*)a.part, a.M, a.S, k, (float*)out);
-    else pw::cover_finish_kernel<<<fb, 256, 0, s>>>((const uint8_t*)a.part, a.M, a.S, (uint8_t*)out);
+    else pw::radius_finish_kernel<<<fb, 256, 0, s>>>(a.part, a.M, a.S, mode, out);
     return launched("dadd_pairwise finish");
 }

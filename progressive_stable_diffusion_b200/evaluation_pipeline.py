@@ -2,8 +2,8 @@
 ``/root/reference/src/pipelines/evaluation/evaluation_pipeline.py`` (``_prepare_conditioning`` :406-461,
 ``_set_delta_scale`` :464-468, ``_ddim_sample_batched`` :471-564, ``_decode_latents`` :567-574, ``GenerationJob`` / ``_collect_jobs``
 :83-89,843-864, the job order, batching and per-class grouping of ``generate_all`` :867-975) - and its scoring: ``evaluate_images`` computes CMMD and improved precision / recall per target class
-(``evaluate_one_run`` :577-839,978-1179) on ``metrics.py``.  A sweep runs ``generate_all`` -> ``group_by_target`` ->
-``evaluate_images``.  FID is not computed: its backbone, torch-fidelity's TF-ported InceptionV3, is not available here.
+(``evaluate_one_run`` :577-839,978-1179), optionally density / coverage, on ``metrics.py``; ``realism_by_class`` scores each
+generated image.  A sweep runs ``generate_all`` -> ``group_by_target`` -> ``evaluate_images`` / ``realism_by_class``.  FID is not computed: its backbone, torch-fidelity's TF-ported InceptionV3, is not available here.
 """
 
 from __future__ import annotations
@@ -147,11 +147,13 @@ def generate_all(module, jobs: Sequence[Tuple[int, float, float]], image_tokens:
 
 @torch.no_grad()
 def evaluate_images(real_by_class: Dict[int, Tensor], fake_by_class: Dict[int, Tensor], clip: "metrics.ClipEmbedder",
-                    vgg: "metrics.VGGFeatures", k: int = 3) -> Dict[object, Dict[str, float]]:
+                    vgg: "metrics.VGGFeatures", k: int = 3, density_coverage: bool = False) -> Dict[object, Dict[str, float]]:
     """CMMD and improved precision / recall of generated against real [0, 1] images, per target class and over all classes.
     ``real_by_class`` / ``fake_by_class``: ``{class: (N, 3, H, W)}`` as ``group_by_target`` returns them.  Returns
     ``{class: {"cmmd", "precision", "recall"}, ..., "all": {...}}``.  A class missing or empty on either side is left out;
-    precision and recall are NaN where a side has k + 1 points or fewer (a k-NN radius needs k other points and more)."""
+    precision and recall are NaN where a side has k + 1 points or fewer (a k-NN radius needs k other points and more).
+    ``density_coverage``: each group also gets ``"density"`` and ``"coverage"`` (Naeem et al. 2020, on the same VGG features
+    and real radii), NaN under the same condition."""
     out: Dict[object, Dict[str, float]] = {}
     feats = {}
     for cls in ALL_MES_CLASSES:
@@ -164,7 +166,27 @@ def evaluate_images(real_by_class: Dict[int, Tensor], fake_by_class: Dict[int, T
         groups.append(("all", tuple(torch.cat([f[i] for f in feats.values()]) for i in range(4))))
     for key, (cr, cf, vr, vf) in groups:
         res = {"cmmd": metrics.cmmd(cr, cf), "precision": float("nan"), "recall": float("nan")}
+        if density_coverage:
+            res["density"] = res["coverage"] = float("nan")
         if min(vr.shape[0], vf.shape[0]) > k + 1:
             res["precision"], res["recall"] = metrics.precision_recall(vr, vf, k)
+            if density_coverage:
+                res["density"], res["coverage"] = metrics.density_coverage(vr, vf, k)
         out[key] = res
+    return out
+
+
+@torch.no_grad()
+def realism_by_class(real_by_class: Dict[int, Tensor], fake_by_class: Dict[int, Tensor], vgg: "metrics.VGGFeatures",
+                     k: int = 3) -> Dict[int, Tensor]:
+    """Realism score (``metrics.realism_scores``) of every generated [0, 1] image against the real images of its own class:
+    ``{class: (N_fake,) CPU float32}``, index n scoring the n-th image of ``fake_by_class[class]`` (``group_by_target``'s
+    order), for ranking or filtering generated images.  A class is left out when either side is missing or empty, or when it
+    has k + 1 real images or fewer."""
+    out: Dict[int, Tensor] = {}
+    for cls in ALL_MES_CLASSES:
+        real, fake = real_by_class.get(cls), fake_by_class.get(cls)
+        if real is None or fake is None or real.shape[0] <= k + 1 or fake.shape[0] == 0:
+            continue
+        out[cls] = metrics.realism_scores(vgg(real), vgg(fake), k).cpu()
     return out

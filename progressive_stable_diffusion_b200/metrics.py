@@ -1,13 +1,16 @@
-"""Image-quality metrics of the evaluation sweep: CMMD and improved precision / recall.
+"""Image-quality metrics of the evaluation sweep: CMMD, improved precision / recall, density / coverage and realism scores.
 
 Replaces the CMMD and precision / recall halves of ``evaluate_one_run`` (reference
-``src/pipelines/evaluation/evaluation_pipeline.py:577-839,978-1179``):
+``src/pipelines/evaluation/evaluation_pipeline.py:577-839,978-1179``), and adds their usual companions:
 
 - ``cmmd``: google-research/cmmd's ``mmd`` over CLIP ViT-L/14-336 embeddings (``ClipEmbedder``);
-- ``precision_recall``: Kynkaanniemi et al. 2019 over VGG16 ``fc2`` features (``VGGFeatures``).
+- ``precision_recall``: Kynkaanniemi et al. 2019 over VGG16 ``fc2`` features (``VGGFeatures``);
+- ``density_coverage``: Naeem et al. 2020 (clovaai/generative-evaluation-prdc) on the same features and real-set radii;
+- ``realism_scores``: the per-image realism score of Kynkaanniemi et al. 2019 (section 5), for ranking generated images.
 
-Both reduce to statistics over all pairs of feature vectors, which ``ops.pairwise_rbf_sum`` / ``ops.knn_radii`` /
-``ops.within_radii`` compute on one fused tcgen05 kernel without materialising the M x N distance matrix.  The ``*_reference``
+All reduce to statistics over all pairs of feature vectors, which ``ops.pairwise_rbf_sum`` / ``ops.knn_radii`` /
+``ops.within_radii`` / ``ops.count_within_radii`` / ``ops.max_radius_ratio`` compute on one fused tcgen05 kernel without
+materialising the M x N distance matrix.  The ``*_reference``
 functions are the same formulas in float64 on whatever device their inputs are on (the tests' yardstick).  FID is not here:
 its backbone is torch-fidelity's TF-ported InceptionV3, which this package cannot restate faithfully.
 """
@@ -33,6 +36,14 @@ IMAGENET_STD = (0.229, 0.224, 0.225)
 # the improved precision / recall metric uses.  The original project's metric code is not available here, so its exact layer
 # choice could not be checked against it.
 VGG_FC2_END = 4
+
+# Realism score (Kynkaanniemi et al. 2019, section 5): the real set is first pruned to the points whose k-NN radius is at most
+# the REALISM_PRUNE_PERCENTILE-th percentile of all radii (linear interpolation, as np.percentile), which drops the half of the
+# balls with the largest radii, so that outliers cannot dominate the max; REALISM_EPS (added to the squared distance) keeps the
+# ratio finite when a generated point lands on a real one.  The original project's metric code is not available here, so these
+# two values could not be checked against it.
+REALISM_EPS = 1e-5
+REALISM_PRUNE_PERCENTILE = 50.0
 
 
 # --------------------------------------------------------------------------------------------- the metrics
@@ -61,6 +72,36 @@ def precision_recall(real_feats: torch.Tensor, fake_feats: torch.Tensor, k: int 
     precision = ops.within_radii(y, x, r_real).float().mean()
     recall = ops.within_radii(x, y, r_fake).float().mean()
     return float(precision), float(recall)
+
+
+def density_coverage(real_feats: torch.Tensor, fake_feats: torch.Tensor, k: int = 3) -> Tuple[float, float]:
+    """Density and coverage (Naeem et al. 2020) on squared Euclidean distances, with the real k-NN radii r2 of
+    ``precision_recall`` and strict ``<`` as in clovaai/generative-evaluation-prdc:
+    density = sum_j #{i : d2(y_j, x_i) < r2_i} / (k N), coverage = #{i : min_j d2(x_i, y_j) < r2_i} / M.  Needs M > k + 1 real
+    and N >= 2 generated points."""
+    x, y = _feats(real_feats), _feats(fake_feats)
+    r_real = ops.knn_radii(x, k)
+    below = torch.nextafter(r_real, torch.full_like(r_real, -float("inf")))      # d2 < r2  <=>  d2 <= the float below r2
+    density = ops.count_within_radii(y, x, below).double().sum() / (k * y.shape[0])
+    coverage = (ops.knn_radii(x, 1, ref=y) < r_real).double().mean()
+    return float(density), float(coverage)
+
+
+def _realism_kept(r_real: torch.Tensor) -> torch.Tensor:
+    """The reals whose radius is at most the REALISM_PRUNE_PERCENTILE-th percentile of all radii."""
+    r = r_real.double()
+    return r <= torch.quantile(r, REALISM_PRUNE_PERCENTILE / 100.0)
+
+
+def realism_scores(real_feats: torch.Tensor, fake_feats: torch.Tensor, k: int = 3) -> torch.Tensor:
+    """(N,) float32 realism score of each generated point (Kynkaanniemi et al. 2019, section 5):
+    R_j = sqrt(max over kept reals i of r2_i / (d2(y_j, x_i) + REALISM_EPS)), the ratio of Euclidean distances, where the
+    kept reals are those with r2_i at most the REALISM_PRUNE_PERCENTILE-th percentile of the radii of the whole real set.
+    R_j >= 1 roughly means y_j lies inside the pruned real manifold.  Needs M > k + 1 real points."""
+    x, y = _feats(real_feats), _feats(fake_feats)
+    r_real = ops.knn_radii(x, k)
+    keep = _realism_kept(r_real)
+    return ops.max_radius_ratio(y, x[keep].contiguous(), r_real[keep].contiguous(), REALISM_EPS).sqrt_()
 
 
 def _sqdist64(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
@@ -92,6 +133,21 @@ def precision_recall_reference(real_feats: torch.Tensor, fake_feats: torch.Tenso
     r_real, r_fake = knn_radii_reference(real_feats, k), knn_radii_reference(fake_feats, k)
     return (float(within_radii_reference(fake_feats, real_feats, r_real).double().mean()),
             float(within_radii_reference(real_feats, fake_feats, r_fake).double().mean()))
+
+
+def density_coverage_reference(real_feats: torch.Tensor, fake_feats: torch.Tensor, k: int = 3) -> Tuple[float, float]:
+    """``density_coverage`` in float64 with the full distance matrix."""
+    r = knn_radii_reference(real_feats, k)
+    inside = _sqdist64(fake_feats, real_feats) < r[None, :]                      # [fake j][real i]
+    return float(inside.double().sum() / (k * fake_feats.shape[0])), float(inside.any(dim=0).double().mean())
+
+
+def realism_scores_reference(real_feats: torch.Tensor, fake_feats: torch.Tensor, k: int = 3) -> torch.Tensor:
+    """``realism_scores`` in float64 with the full distance matrix."""
+    r = knn_radii_reference(real_feats, k)
+    keep = _realism_kept(r)
+    ratio = r[keep][None, :] / (_sqdist64(fake_feats, real_feats[keep]) + REALISM_EPS)
+    return ratio.amax(dim=1).sqrt()
 
 
 # --------------------------------------------------------------------------------------------- backbones

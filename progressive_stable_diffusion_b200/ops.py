@@ -512,7 +512,7 @@ def adamw_step_(p: torch.Tensor, g: torch.Tensor, m: torch.Tensor, v: torch.Tens
 
 
 # --------------------------------------------------------------------------------------------- evaluation metrics
-RBF_SUM, KNN, COVER = 0, 1, 2
+RBF_SUM, KNN, COVER, COUNT, RATIO_MAX = 0, 1, 2, 3, 4
 
 
 def _features(*ts: torch.Tensor) -> None:
@@ -546,17 +546,35 @@ def pairwise_rbf_sum(x: torch.Tensor, y: Optional[torch.Tensor], gamma: float) -
     return _pairwise(x, y, RBF_SUM, torch.empty((), dtype=torch.float64, device=x.device), gamma=gamma)
 
 
-def knn_radii(x: torch.Tensor, k: int) -> torch.Tensor:
+def knn_radii(x: torch.Tensor, k: int, ref: Optional[torch.Tensor] = None) -> torch.Tensor:
     """(M,) float32: the squared distance from each row of x to its k-th nearest OTHER row (1 <= k <= 16, M > k + 1): the
-    manifold radii of improved precision / recall (Kynkaanniemi et al. 2019)."""
-    _features(x)
-    return _pairwise(x, None, KNN, torch.empty(x.shape[0], dtype=torch.float32, device=x.device), k=k)
+    manifold radii of improved precision / recall (Kynkaanniemi et al. 2019).  With ``ref`` (N, D): the k-th smallest squared
+    distance from each row of x to the rows of ref (N > k), nothing excluded (k = 1: the nearest-neighbour distance)."""
+    _features(x, *(() if ref is None else (ref,)))
+    return _pairwise(x, ref, KNN, torch.empty(x.shape[0], dtype=torch.float32, device=x.device), k=k)
 
 
-def within_radii(q: torch.Tensor, ref: torch.Tensor, radii: torch.Tensor) -> torch.Tensor:
-    """(M,) bool: whether each row of q lies in at least one ball |q_i - ref_j|^2 <= radii[j] (improved precision / recall)."""
+def _radii(q: torch.Tensor, ref: torch.Tensor, radii: torch.Tensor) -> None:
     _features(q, ref)
     _cuda(radii)
     if radii.dtype != torch.float32 or radii.shape != (ref.shape[0],) or not radii.is_contiguous():
         raise _lib.DaddError(f"radii must be a contiguous float32 ({ref.shape[0]},) tensor")
+
+
+def within_radii(q: torch.Tensor, ref: torch.Tensor, radii: torch.Tensor) -> torch.Tensor:
+    """(M,) bool: whether each row of q lies in at least one ball |q_i - ref_j|^2 <= radii[j] (improved precision / recall)."""
+    _radii(q, ref, radii)
     return _pairwise(q, ref, COVER, torch.empty(q.shape[0], dtype=torch.bool, device=q.device), radii=radii)
+
+
+def count_within_radii(q: torch.Tensor, ref: torch.Tensor, radii: torch.Tensor) -> torch.Tensor:
+    """(M,) int32: for each row of q, the number of balls |q_i - ref_j|^2 <= radii[j] it lies in (density, Naeem et al. 2020)."""
+    _radii(q, ref, radii)
+    return _pairwise(q, ref, COUNT, torch.empty(q.shape[0], dtype=torch.int32, device=q.device), radii=radii)
+
+
+def max_radius_ratio(q: torch.Tensor, ref: torch.Tensor, radii: torch.Tensor, eps: float) -> torch.Tensor:
+    """(M,) float32: max over j of radii[j] / (|q_i - ref_j|^2 + eps), eps finite and > 0, 0 when no ratio is positive (the
+    squared realism score of Kynkaanniemi et al. 2019)."""
+    _radii(q, ref, radii)
+    return _pairwise(q, ref, RATIO_MAX, torch.empty(q.shape[0], dtype=torch.float32, device=q.device), gamma=eps, radii=radii)

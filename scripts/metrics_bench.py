@@ -1,6 +1,8 @@
-"""Time the fused pairwise kernel (ops.knn_radii / within_radii / pairwise_rbf_sum) against the torch fp32 path
-(cdist + topk / exp().mean()) on the evaluation metrics' sizes: a LIMUC-sized real set of 11 264 images against itself
-(IPR radii, VGG16 fc2 width 4096), 2 400 generated against it (IPR coverage), and CMMD's CLIP width 768.
+"""Time the fused pairwise kernel (ops.knn_radii / within_radii / pairwise_rbf_sum / count_within_radii / max_radius_ratio)
+against the torch fp32 path (cdist + topk / exp().mean() / a comparison or ratio reduced over the rows) on the evaluation
+metrics' sizes: a LIMUC-sized real set of 11 264 images against itself (IPR radii, VGG16 fc2 width 4096), 2 400 generated
+against it (IPR coverage, density counts), 2 400 generated against the kept half of it (realism scores), and CMMD's CLIP
+width 768.
 
     python scripts/metrics_bench.py [--reps 10]
 
@@ -40,7 +42,7 @@ def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=10)
     args = ap.parse_args()
-    from progressive_stable_diffusion_b200 import ops
+    from progressive_stable_diffusion_b200 import metrics, ops
     assert torch.cuda.is_available(), "needs a CUDA device"
     try:
         q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
@@ -55,6 +57,8 @@ def main() -> None:
     cfake = torch.nn.functional.normalize(torch.randn(2400, 768, device="cuda", generator=g) + 0.02, dim=1)
     k, gamma = 3, 1.0 / 200.0
     r_real = ops.knn_radii(real, k)
+    keep = metrics._realism_kept(r_real)
+    kept, r_kept = real[keep].contiguous(), r_real[keep].contiguous()
 
     def torch_radii():
         d = torch.cdist(real, real).square_()
@@ -70,6 +74,13 @@ def main() -> None:
         ("CMMD sum 11264 x 2400, D 768", 11264, 2400, 768, lambda: ops.pairwise_rbf_sum(creal, cfake, gamma),
          lambda: torch.exp(-gamma * torch.cdist(creal, cfake).square_()).sum(),
          lambda a, b: f"relative diff {abs(a.item() - b.item()) / b.item():.2e}"),
+        ("density counts 2400 x 11264, D 4096", 2400, 11264, 4096, lambda: ops.count_within_radii(fake, real, r_real),
+         lambda: (torch.cdist(fake, real).square_() <= r_real[None]).sum(1),
+         lambda a, b: f"{int((a != b).sum())} of {a.numel()} counts differ, max |diff| {int((a - b).abs().max())}"),
+        (f"realism 2400 x {kept.shape[0]} kept, D 4096", 2400, kept.shape[0], 4096,
+         lambda: ops.max_radius_ratio(fake, kept, r_kept, metrics.REALISM_EPS),
+         lambda: (r_kept[None] / (torch.cdist(fake, kept).square_() + metrics.REALISM_EPS)).amax(1),
+         lambda a, b: f"max relative diff {((a - b).abs() / b).max().item():.2e}"),
     ]
     print(f"torch.backends.cuda.matmul.allow_tf32 = {torch.backends.cuda.matmul.allow_tf32} (cdist runs in fp32)")
     for name, m, n, d, ours, ref, agree in work:
@@ -78,7 +89,7 @@ def main() -> None:
         flops = 3 * 2.0 * m * n * d
         print(f"{name}: kernel {t0 * 1e3:.2f} ms ({flops / t0 / 1e12:.0f} TFLOP/s three-pass, {flops / t0 / TF32_PEAK * 100:.1f} % of "
               f"the tf32 peak), peak mem {m0 / 1e6:.0f} MB | torch fp32 {t1 * 1e3:.2f} ms, peak mem {m1 / 1e6:.0f} MB | "
-              f"speed-up {t1 / t0:.2f}x | {agree(o0.double() if o0.is_floating_point() else o0, o1.double() if o1.is_floating_point() else o1)}")
+              f"speed-up {t1 / t0:.2f}x | {agree(o0.double() if o0.is_floating_point() else o0.long(), o1.double() if o1.is_floating_point() else o1.long())}")
 
 
 if __name__ == "__main__":
